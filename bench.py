@@ -7,8 +7,9 @@ Contract (driver): prints ONE JSON line on rank 0.  ``value`` = whole-job region
 resident in HBM; ``e2e`` = the same metric through the public module API with HOST (pinned) inputs, the
 host->device copies and a device->host read of the loss inside the timed region; ``roofline`` = the
 Chebyshev SpMM (the forward's 18 recurrence launches at cfg3) timed alone with CUDA events against the
-measured HBM peak; ``cpu_baseline`` = the UNMODIFIED reference modules (``baseline/_ref``, staged by build(); the
-oracle port if absent) on this box's host cores on a bounded sample.  ``--impl reference`` times only that CPU path.
+measured HBM peak; ``cpu_baseline`` = the UNMODIFIED reference modules (``oracle/_ref``, staged by build() or
+``oracle/stage_reference.py``; the oracle port if absent) on the host's cores on a bounded sample.  ``--impl reference``
+times only that CPU path.  ``--dump-outputs DIR`` writes what the last timed step computed (see ``dump_outputs``).
 
 Default workload: cfg3 = BASELINE.json configs[2] (4096 regions, 3 graphs, K=3, seq_len=12, batch 64 per
 GPU, fp32) -- the configuration BASELINE.json's metric quotes the SpMM HBM figure on, and the largest fp32
@@ -50,7 +51,15 @@ def parse_args():
     ap.add_argument("--cuda-graph", action="store_true",
                     help="replay the step from a captured CUDA graph (stmgcn_b200.graphs.GraphedStep); measured gain "
                          "at cfg3 is ~1 %% -- the step is GPU-bound, not launch-bound -- so eager is the default")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output, loss and parameter gradients of the last timed step "
+                         "as DIR/<name>.npy (written by rank 0: its own output and loss, the all-reduced gradients)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -120,6 +129,30 @@ class ClockSampler:
         return out
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(path, out, loss, model):
+    """Write what a step hands back to its caller -- the model output, the MSE loss and every parameter gradient -- as
+    float32 ``path/out.npy``, ``path/loss.npy`` and ``path/grad.<parameter name>.npy``.  The inputs are a pure function of
+    the arguments, so two builds can be compared file by file.  An output too large for the 64 MB budget is written as
+    the fixed sample ``out.reshape(-1)[::stride]``.  With several GPUs, rank 0 calls this: ``out`` and ``loss`` are its
+    own shard of the batch, the gradients are the all-reduced means every rank holds."""
+    import numpy as np
+    arrays = {"loss": loss.detach().float().cpu().numpy()}
+    arrays.update({"grad." + k: p.grad.detach().float().cpu().numpy() for k, p in model.named_parameters()})
+    o = out.detach().float().cpu().numpy()
+    room = DUMP_BUDGET_BYTES - sum(a.nbytes for a in arrays.values())
+    if room <= 0:
+        raise RuntimeError(f"--dump-outputs: the gradients alone exceed {DUMP_BUDGET_BYTES} bytes")
+    if o.nbytes > room:
+        o = o.reshape(-1)[::-(-o.nbytes // room)]
+    arrays["out"] = o
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def spmm_algorithmic_bytes(n, nnz, f_total, k_order, elem=4):
     """SURVEY.md section 8(d): per GCN call K*CSR + N*F*e*(3K-1)."""
     csr = nnz * 8 + (n + 1) * 4
@@ -129,12 +162,12 @@ def spmm_algorithmic_bytes(n, nnz, f_total, k_order, elem=4):
 # ---------------------------------------------------------------------------------------------------
 # reference arm: the oracle port (dense supports + nn.LSTM, the reference's algorithm) on host cores
 # ---------------------------------------------------------------------------------------------------
-REF_DIR = os.path.join(REPO, "baseline", "_ref")
+REF_DIR = os.path.join(REPO, "oracle", "_ref")
 
 
 def _reference_modules():
-    """The UNMODIFIED reference's ``GCN`` / ``STMGCN`` modules from ``baseline/_ref`` (staged by
-    ``__graft_entry__.build()``), imported under private names so they can never shadow the repo's drop-in modules.
+    """The UNMODIFIED reference's ``GCN`` / ``STMGCN`` modules from ``oracle/_ref`` (staged by
+    ``oracle/stage_reference.py``), imported under private names so they can never shadow the repo's drop-in modules.
     Returns None when the directory was not staged (then the oracle port is timed instead)."""
     if not os.path.exists(os.path.join(REF_DIR, "STMGCN.py")):
         return None
@@ -162,10 +195,10 @@ def _reference_modules():
 def cpu_reference_run(w, steps, warmup, sample_batch=None, log=None, step_budget_s=6.0):
     """Time the reference's CPU implementation of the path on the host cores.
 
-    kind "reference": the unmodified reference modules from ``baseline/_ref`` -- ``Adj_Preprocessor.process`` (dense
+    kind "reference": the unmodified reference modules from ``oracle/_ref`` -- ``Adj_Preprocessor.process`` (dense
     supports, GCN.py:57-97), ``ST_MGCN.forward`` (STMGCN.py:100-119), ``nn.MSELoss``, ``backward`` -- exactly the step of
     ``Model_Trainer.py:35-41`` without the optimizer.  kind "port": the oracle's dense restatement (same algorithm, same
-    torch ops) when ``baseline/_ref`` is absent.
+    torch ops) when ``oracle/_ref`` is absent.
 
     Thread count: "all the host threads it can use" is calibrated, not assumed -- on the GPU boxes os.cpu_count()
     reports 128 logical CPUs but running 128 intra-op threads is ~50x SLOWER than 16-32 (measured: 64 s vs 1.1 s for a
@@ -241,9 +274,9 @@ def cpu_reference_run(w, steps, warmup, sample_batch=None, log=None, step_budget
         model_name = [l.split(":")[1].strip() for l in open("/proc/cpuinfo") if l.startswith("model name")][0]
     except Exception:
         model_name = "unknown"
-    what = ("the UNMODIFIED reference modules (baseline/_ref: Adj_Preprocessor.process dense supports, ST_MGCN.forward, "
+    what = ("the UNMODIFIED reference modules (oracle/_ref: Adj_Preprocessor.process dense supports, ST_MGCN.forward, "
             "MSELoss, backward)" if kind == "reference" else
-            "the oracle port (dense supports + nn.LSTM, as the reference executes; baseline/_ref not staged)")
+            "the oracle port (dense supports + nn.LSTM, as the reference executes; oracle/_ref not staged)")
     return dict(value=value, unit=UNIT, cores=best_c, kind=kind,
                 sample=f"{w.name} shapes with batch {sample_batch} (of {w.batch}), {steps} timed step(s) after "
                        f"{warmup} warm-up, fwd+MSE+bwd through {what}, "
@@ -309,6 +342,8 @@ def run_ours(args, w):
 
     use_graph = args.cuda_graph
     launches_per_step = None
+    last = {}                              # output and loss of the latest step (--dump-outputs); detached, so the
+                                           # step's autograd graph and LSTM tape are freed as before
     if use_graph:
         # one eager step to count this library's launches, then capture fwd + loss + bwd (+ all-reduce) once
         l0 = _lib.launch_count()
@@ -321,6 +356,7 @@ def run_ours(args, w):
         def step(x, y):
             loss = gstep(x, y)
             bucket.all_reduce_mean_()          # the one collective of the step stays outside the graph (NCCL, eager)
+            last.update(out=gstep.out, loss=loss)
             return loss
     else:
         def step(x, y):
@@ -329,6 +365,7 @@ def run_ours(args, w):
             loss = crit(out, y)
             loss.backward()
             bucket.all_reduce_mean_()
+            last.update(out=out.detach(), loss=loss.detach())
             return loss
 
     ms_step_local = [0.0]                  # this rank's own device time per step of the last timed() call
@@ -362,6 +399,8 @@ def run_ours(args, w):
     ms_total = timed(lambda: step(x_d, y_d), args.steps)
     launches = (_lib.launch_count() - l0) // args.steps if launches_per_step is None else launches_per_step
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["out"], last["loss"], model)
     ms_step = ms_total / args.steps
     units = b * world * w.n_regions * w.seq_len
     value = units / (ms_step * 1e-3)

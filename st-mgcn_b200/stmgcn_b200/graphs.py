@@ -38,20 +38,20 @@ class GraphedStep:
         torch.cuda.synchronize()
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
-            self.loss = self._eager()
+            self.out, self.loss = self._eager()
 
-    def _eager(self) -> torch.Tensor:
+    def _eager(self):
         self.bucket.zero_()
         out = self.model(obs_seq=self.x, sta_adj_list=self.supports)
         loss = self.criterion(out, self.y)
         loss.backward()
         if self.all_reduce:
             self.bucket.all_reduce_mean_()
-        return loss
+        return out, loss
 
     def __call__(self, x: Optional[torch.Tensor] = None, y: Optional[torch.Tensor] = None) -> torch.Tensor:
         """Copy the batch into the static buffers (host or device source) and replay. Returns the loss tensor
-        (static buffer: read it before the next call)."""
+        (static buffer: read it before the next call); the replay's model output is the static buffer ``self.out``."""
         if x is not None and tuple(x.shape) != tuple(self.x.shape):
             # a batch of another size (the reference's DataLoader yields one short last batch, Data_Container.py:122):
             # shapes are baked into the captured graph, so this batch runs eagerly

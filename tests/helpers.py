@@ -12,11 +12,19 @@ TOL = 1e-4          # BASELINE.json north_star: "within 1e-4 relative fp32" (max
 
 
 def load_golden(name):
-    blob = np.load(os.path.join(GOLDEN, name + ".npz"))
+    """A fixture of oracle/make_golden.py: ``<name>.npz``, continued in ``<name>.1.npz``, ... when it is too large for
+    one file.  Returns the meta dict, parameters, gradients, supports, adjacencies and a dict of every stored array."""
+    paths = [os.path.join(GOLDEN, name + ".npz")]
+    while os.path.exists(os.path.join(GOLDEN, f"{name}.{len(paths)}.npz")):
+        paths.append(os.path.join(GOLDEN, f"{name}.{len(paths)}.npz"))
+    blob = {}
+    for path in paths:
+        with np.load(path) as part:
+            blob.update((key, part[key]) for key in part.files)
     n, m, k, t, b, c, hid, layers, gcn_hid = [int(v) for v in blob["meta"]]
     meta = dict(n=n, m=m, k=k, t=t, b=b, c=c, hid=hid, layers=layers, gcn_hid=gcn_hid)
-    params = {key[len("param."):]: torch.from_numpy(blob[key]) for key in blob.files if key.startswith("param.")}
-    grads = {key[len("grad."):]: blob[key] for key in blob.files if key.startswith("grad.")}
+    params = {key[len("param."):]: torch.from_numpy(blob[key]) for key in blob if key.startswith("param.")}
+    grads = {key[len("grad."):]: blob[key] for key in blob if key.startswith("grad.")}
     supports = [torch.from_numpy(blob[f"supports.{g}"]) for g in range(m)]
     adjs = [torch.from_numpy(blob[f"adj.{g}"]) for g in range(m)]
     return meta, params, grads, supports, adjs, blob

@@ -2,13 +2,17 @@
 ``GCN`` / ``STMGCN`` modules (BASELINE.json north_star: "Main.py and Model_Trainer.py run unchanged"; SURVEY.md section 4
 "drop-in" row, section 8(c) bullet 2).
 
-The five reference files are staged, byte for byte, under ``baseline/_ref/`` by ``__graft_entry__.build()`` in the build
-container (git-ignored, shipped to the GPU box by gpurun).  The script is driven through its own command line only
-(``--device``, ``--dates``): nothing is patched, the hard-coded ``epoch = 100`` (``Main.py:11``) runs with the trainer's
-own early stopping (``Model_Trainer.py:54-60``) on a synthetic ``./data/data_dict.npz`` (the dataset is not shipped,
-``Main.py:9``): ``taxi (T,58,1)`` plus three ``(58,58)`` adjacencies.
+The five reference files are staged, byte for byte, under the git-ignored ``oracle/_ref/`` by
+``oracle/stage_reference.py`` (``__graft_entry__.build()`` runs it when it finds a checkout of the original) and
+checked against their SHA-256 in ``tests/golden/reference_sha256.json``.  The original sources are not part of this
+repository, so the test skips where nothing was staged.  The script is driven through its own command line only
+(``--device``, ``--dates``): nothing is patched, the hard-coded ``epoch = 100`` (``Main.py:11``) runs with the
+trainer's own early stopping (``Model_Trainer.py:54-60``) on a synthetic ``./data/data_dict.npz`` (the dataset is not
+shipped, ``Main.py:9``): ``taxi (T,58,1)`` plus three ``(58,58)`` adjacencies.
 """
+import hashlib
 import io
+import json
 import os
 import re
 import runpy
@@ -21,7 +25,7 @@ import torch
 
 pytestmark = pytest.mark.gpu
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(REPO, "baseline", "_ref")
+REF = os.path.join(REPO, "oracle", "_ref")
 
 
 def _write_dataset(path, hours=24 * 16, n=58, seed=0):
@@ -42,12 +46,16 @@ def _write_dataset(path, hours=24 * 16, n=58, seed=0):
 
 
 @pytest.mark.skipif(not os.path.exists(os.path.join(REF, "Main.py")),
-                    reason="baseline/_ref not staged (run __graft_entry__.build() where /root/reference exists)")
+                    reason="original project not staged (build() stages it from a checkout it finds, or run "
+                           "python oracle/stage_reference.py <its checkout>)")
 def test_reference_main_runs_unchanged_on_the_b200_modules(tmp_path):
     from stmgcn_b200 import _lib
-    # byte-identical to what build() staged: the test must not run a doctored script
-    for name in ("Main.py", "Model_Trainer.py", "Data_Container.py"):
-        assert os.path.getsize(os.path.join(REF, name)) > 0
+    # the staged files are the unmodified original (SHA-256 of commit 5ee7e17): the test must not run a doctored script
+    with open(os.path.join(REPO, "tests", "golden", "reference_sha256.json")) as fh:
+        digests = json.load(fh)
+    for name, digest in digests.items():
+        with open(os.path.join(REF, name), "rb") as fh:
+            assert hashlib.sha256(fh.read()).hexdigest() == digest, f"oracle/_ref/{name} differs from the original"
     _write_dataset(str(tmp_path / "data" / "data_dict.npz"))
     saved_path, saved_argv, saved_cwd = list(sys.path), list(sys.argv), os.getcwd()
     saved_mods = {k: sys.modules.pop(k) for k in ("GCN", "STMGCN", "Model_Trainer", "Data_Container") if k in sys.modules}
