@@ -60,18 +60,4 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
-// streaming (read-once) 128-bit load that does not pollute L1
-__device__ __forceinline__ float4 ld_stream4(const float* p) {
-    float4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w)
-                 : "l"(p));
-    return r;
-}
-__device__ __forceinline__ void st_stream4(float* p, const float4& v) {
-    asm volatile("st.global.L1::no_allocate.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y),
-                 "f"(v.z), "f"(v.w)
-                 : "memory");
-}
-
 }  // namespace stmgcn

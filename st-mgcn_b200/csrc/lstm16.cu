@@ -10,8 +10,8 @@
 //        (32 consecutive rows, the same 4 units) touch ONE contiguous 512-byte run per access.  (With 8-unit groups every
 //        access was 16 bytes at a 32-byte stride: 32 half-used sectors and ~22 L1 data-pipe wavefronts per request; ncu
 //        showed the L1 data pipe -- tensor-core operand reads + LSU -- at 77 % (forward) / 90 % (backward) of its peak.)
-// 4 + 4 bytes per (row, unit, layer-step) instead of 4 + 4 + 16 with the gate tape of the first generation
-// (lstm_tc.cu): 4.8 GB instead of 14.5 GB per graph branch at BASELINE configs[2], and configs[4] fits.
+// 4 + 4 bytes per (row, unit, layer-step) instead of 4 + 4 + 16 with the gate tape of the first-generation (3xTF32)
+// kernels: 4.8 GB instead of 14.5 GB per graph branch at BASELINE configs[2], and configs[4] fits.
 //
 // forward kernel (one launch per layer-step, persistent, one CTA per SM):
 //   producer warp : loads the layer's weight image ONCE (resident for the whole launch: [256 gate cols][64 k] bf16 tiles,

@@ -13,8 +13,8 @@ int32_t launch_proj_bwd_tc(const float* d_out, const float* out_act, int act, in
                            float* dz_out, float* dbias, float* u, int64_t stride_u, cudaStream_t st);
 int32_t launch_pack_image(const float* src, int n_rows, int k_cols, int64_t rs, int64_t cs, float* img, int tile_rows,
                           cudaStream_t st);
-int32_t launch_wgrad_tc(const float* seg0, const float* seg1, const float* h0, int shift1, const float* da, int n,
-                        float* dwp, int kd, int t_len, int64_t rows, cudaStream_t st);
+int32_t launch_proj_tc_wgrad(const float* seg0, const float* seg1, const float* dz, int64_t rows, float* dw,
+                             cudaStream_t st);
 }
 
 namespace {
@@ -238,7 +238,7 @@ int32_t stmgcn_proj_bwd(const float* s, int64_t stride_k, int32_t ks, int64_t ro
     cudaStream_t st = (cudaStream_t)stream;
     if (wimg_t && u && d_out && proj_tc_applicable(ks, p, q, s, out, d_out) && aligned16(dz_work) && aligned16(u) &&
         stride_k % 4 == 0 && stride_u % 4 == 0) {
-        // tcgen05 path: dZ + bias gradient + U in one kernel, then dW per 128-row block of W (proj_tc.cu, lstm_tc.cu)
+        // tcgen05 path (proj_tc.cu): dZ + bias gradient + U in one kernel, then dW per 128-row block of W
         // U has 64*ks columns; one launch produces up to 256 of them (supports 0..3), a second one the rest (it re-forms
         // dZ in its loader but neither stores it nor accumulates the bias gradient again)
         if (int32_t rc = launch_proj_bwd_tc(d_out, out, act, rows, ks < 4 ? ks : 4, wimg_t, dz_work, dbias, u, stride_u, st)) return rc;
@@ -247,12 +247,9 @@ int32_t stmgcn_proj_bwd(const float* s, int64_t stride_k, int32_t ks, int64_t ro
                                                 u + 4 * stride_u, stride_u, st))
                 return rc;
         for (int k0 = 0; k0 < ks; k0 += 2) {
-            const bool two = k0 + 1 < ks;
-            const float* s0 = two ? s + (int64_t)k0 * stride_k : nullptr;
-            const float* s1 = s + (int64_t)(two ? k0 + 1 : k0) * stride_k;
-            if (int32_t rc = launch_wgrad_tc(s0, s1, nullptr, 0, dz_work, 64, dw + (int64_t)k0 * 64 * 64, two ? 128 : 64, 1,
-                                             rows, st))
-                return rc;
+            const float* s0 = s + (int64_t)k0 * stride_k;
+            const float* s1 = k0 + 1 < ks ? s0 + stride_k : nullptr;     // nullptr: the 64-row tail block of W
+            if (int32_t rc = launch_proj_tc_wgrad(s0, s1, dz_work, rows, dw + (int64_t)k0 * 64 * 64, st)) return rc;
         }
         return 0;
     }

@@ -1,12 +1,7 @@
-// Blackwell (sm_100a) primitives used by the tensor-core kernels: mbarrier, 1-D bulk async copy (TMA unit,
-// SASS UBLKCP), tcgen05 (alloc / mma kind::tf32 / commit / ld / fences), UMMA descriptors.
-//
-// Precision scheme "3xTF32": every fp32 operand v is split into hi = v with the low 13 mantissa bits cleared
-// (exactly representable in tf32, so the tensor core's own fp32->tf32 conversion cannot change it) and
-// lo = v - hi (exact in fp32; <= 13 significant bits, again masked to tf32).  A.B is accumulated in fp32
-// TMEM as Ahi.Bhi + Alo.Bhi + Ahi.Blo; the dropped Alo.Blo term is ~2^-22 relative.  Measured against the
-// fp64 oracle this keeps the LSTM within ~2e-6 of the exact-fp32 path (the 1e-4 parity bar forbids
-// single-pass TF32, SURVEY.md section 0.5).
+// Blackwell (sm_100a) primitives shared by the tensor-core kernels (lstm16.cu through tc16.cuh, proj_tc.cu): mbarrier
+// and bounded waits, 1-D bulk async copy (TMA unit, SASS UBLKCP), L2 prefetch, wide global stores / reductions,
+// tcgen05 (alloc / commit / ld / fences), the elected single issuing thread and the 128-byte-swizzle UMMA descriptors.
+// The MMA instructions themselves live with their precision scheme: kind::f16 in tc16.cuh, kind::tf32 in proj_tc.cu.
 #pragma once
 #include "common.cuh"
 
@@ -14,12 +9,6 @@ namespace stmgcn {
 namespace tc {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// ---- tf32 split ---------------------------------------------------------------------------------------
-__device__ __forceinline__ float tf32_hi(float v) { return __uint_as_float(__float_as_uint(v) & 0xffffe000u); }
-__device__ __forceinline__ float tf32_lo(float v, float hi) {
-    return __uint_as_float(__float_as_uint(v - hi) & 0xffffe000u);
-}
 
 // ---- mbarrier -----------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -71,7 +60,9 @@ __device__ __forceinline__ void mbar_wait_polite(uint64_t* bar, uint32_t parity)
     __trap();
 }
 // Optional wait-time accounting (built with -DSTMGCN_TC_PROFILE): cycles each role spends blocked on each barrier
-// class, summed per launch into g_tc_prof[slot]; slot = role*4 + barrier class.  Read with stmgcn_dbg_tc_prof().
+// class, summed per launch into g_tc_prof[slot]; slot = role*4 + barrier class.  The library is built without relocatable
+// device code, so every translation unit has its own g_tc_prof: the instrumented kernels are lstm16.cu's, read with
+// stmgcn_dbg_tc_prof16() (tools/tc_role_profile16.py).
 #ifdef STMGCN_TC_PROFILE
 __device__ unsigned long long g_tc_prof[64];
 struct WaitProf {
@@ -107,7 +98,6 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
                  : "memory");
 }
 
-// L2 prefetch of a contiguous global range (no registers, no shared memory; SASS UBLKPF)
 // One elected lane of a fully converged warp.  Guarding the single-thread tcgen05 / TMA / mbarrier instructions with this
 // instead of `lane == 0` matters: ptxas cannot prove `lane == 0` selects one thread, and wraps EVERY uniform-datapath
 // instruction (UTCHMMA, UTCBAR, UBLKCP, UTMALDG) in an ELECT / BRA.U.ANY serialisation loop -- ~10 extra instructions and
@@ -128,6 +118,7 @@ __device__ __forceinline__ void st_global_v8(void* dst, const uint32_t* v) {
 __device__ __forceinline__ void red_add_f32x4(float4* dst, const float4& v) {
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
+// L2 prefetch of a contiguous global range (no registers, no shared memory; SASS UBLKPF)
 __device__ __forceinline__ void prefetch_l2(const void* gmem, uint32_t bytes) {
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gmem), "r"(bytes) : "memory");
 }
@@ -141,40 +132,9 @@ __device__ __forceinline__ void tmem_alloc(uint32_t* smem_slot, uint32_t ncols) 
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {      // same warp that allocated
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
-// ---- TMA tensor stores (shared -> global through a CUtensorMap, bulk async-group completion) ----
-__device__ __forceinline__ void tma_store_2d(const void* tmap, uint32_t smem_addr, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-                 :: "l"(tmap), "r"(smem_addr), "r"(c0), "r"(c1) : "memory");
-}
-// TMA tensor load (global -> shared through a CUtensorMap), completion (bytes) on an mbarrier
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* tmap, int c0, int c1, uint64_t* bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 :: "r"(smem_u32(smem_dst)), "l"(tmap), "r"(smem_u32(bar)), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void bulk_commit_group() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// the issuing thread's bulk groups have finished READING shared memory (the staging tile may be overwritten)
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-// programmatic dependent launch: the next kernel of the stream may start its prologue (barrier init, TMEM allocation)
-// on SMs this grid has already left; pdl_wait() blocks until the previous grid has completed and flushed its memory
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem] . B[smem], tf32 inputs, fp32 accumulate; one thread issues for the CTA.
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                         uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        :
-        : "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
 // all previously issued MMAs of this thread complete -> one arrival on the mbarrier
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -215,15 +175,6 @@ __device__ __forceinline__ uint64_t smem_desc_k_sw128(uint32_t smem_addr) {
     d |= (uint64_t)2 << 61;                              // layout type SWIZZLE_128B [61,64)
     return d;
 }
-// kind::tf32, fp32 accumulate, M x N tile; mn_major = 0: A and B K-major, 1: both MN-major
-__host__ __device__ constexpr uint32_t idesc_tf32(int m, int n, int mn_major = 0) {
-    return (1u << 4)                               // c_format  = F32
-           | (2u << 7)                             // a_format  = TF32
-           | (2u << 10)                            // b_format  = TF32
-           | ((uint32_t)(mn_major & 1) << 15)      // a_major
-           | ((uint32_t)(mn_major & 1) << 16)      // b_major
-           | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
 // MN-major operand, 128-byte swizzle.  Canonical layout (cute/atom/mma_traits_sm100.hpp, in 16-byte units):
 // ((8,n),(8,k)) : ((1,LBO),(8,SBO)) -- a 1024-byte atom holds 32 consecutive M/N elements (one 128-byte row)
 // for each of 8 consecutive K; LBO = byte distance between atoms along M/N, SBO = between atoms along K.
@@ -236,20 +187,6 @@ __device__ __forceinline__ uint64_t smem_desc_mn_sw128(uint32_t smem_addr, uint3
     d |= (uint64_t)1 << 46;
     d |= (uint64_t)layout_type << 61;
     return d;
-}
-// MN-major tile for 32-bit operands: layout type SWIZZLE_128B_BASE32B (1), Swizzle<2,5,2> on the byte address:
-// atoms of 128 B (32 consecutive M/N elements) x 4 K-rows = 512 B; inside an atom the 32-byte chunk index is XORed
-// with the K-row index.  Atoms are laid out [mn atom][k atom]: LBO = (k_rows/4)*512 bytes, SBO = 512 bytes.
-__host__ __device__ __forceinline__ uint32_t mn32_offset(uint32_t q /*float4 index along M/N*/, uint32_t k,
-                                                         uint32_t k_rows) {
-    const uint32_t atom_mn = q >> 3, c16 = q & 7;            // 8 float4 per 128-byte row
-    const uint32_t atom_k = k >> 2, kr = k & 3;
-    return atom_mn * (k_rows >> 2) * 512u + atom_k * 512u + kr * 128u + ((((c16 >> 1) ^ kr) & 3u) << 5) + ((c16 & 1u) << 4);
-}
-
-// byte offset of element (row, k) inside a [rows][32 fp32] K-major tile with the 128-byte swizzle
-__host__ __device__ __forceinline__ uint32_t sw128_offset(uint32_t row, uint32_t k) {
-    return row * 128u + ((((k >> 2) ^ (row & 7u)) & 7u) << 4) + ((k & 3u) << 2);
 }
 
 }  // namespace tc

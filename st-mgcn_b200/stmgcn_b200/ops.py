@@ -162,33 +162,49 @@ def adjoint_stack_(sset: SupportSet, u: torch.Tensor) -> torch.Tensor:
     return acc
 
 
-_PROJ_CACHE: "OrderedDict" = OrderedDict()
+_IMAGE_CACHE_SIZE = 24
+_PROJ_IMAGES: "OrderedDict" = OrderedDict()
+_LSTM16_IMAGES: "OrderedDict" = OrderedDict()
+
+
+def _cached_images(store: "OrderedDict", params: Sequence[torch.Tensor], extra: tuple, pack, usable=None) -> dict:
+    """The dict ``pack()`` returns (operand images of ``params``, packed on the current stream), cached in the LRU ``store``
+    on storage + in-place version of every parameter and ``extra``: re-packed only after an optimizer step changed them,
+    or when ``usable(hit)`` rejects the hit.  During CUDA-graph capture the cache is bypassed so the pack kernels become
+    part of the graph (replays see updated weights)."""
+    capturing = torch.cuda.is_current_stream_capturing()
+    key = tuple((w.data_ptr(), w._version) for w in params) + extra + (str(params[0].device),)
+    if not capturing:
+        hit = store.get(key)
+        if hit is not None and (usable is None or usable(hit)):
+            store.move_to_end(key)
+            torch.cuda.current_stream().wait_event(hit["event"])
+            return hit
+    entry = pack()
+    if not capturing:
+        entry["event"] = torch.cuda.Event()
+        entry["event"].record()
+        entry["keep"] = list(params)          # keeps the storages alive: a recycled data_ptr can never alias the key
+        store[key] = entry
+        while len(store) > _IMAGE_CACHE_SIZE:
+            store.popitem(last=False)
+    return entry
 
 
 def _proj_images(w: torch.Tensor, ks: int, p: int, need_bwd: bool):
-    """tcgen05 operand images of the projection weights (p = q = 64, ks <= 8), or (None, None).  Cached on the
-    parameter's storage + in-place version (re-packed only after an optimizer step; bypassed during CUDA-graph capture so
-    the pack kernels are part of the graph)."""
+    """tcgen05 operand images (forward, backward) of the projection weights (p = q = 64, ks <= 8), or (None, None).
+    The backward image is packed only when ``need_bwd``; an entry without it is re-packed when a later call needs it."""
     if lstm_path() != "tc" or p != 64 or w.shape[1] != 64 or ks > 8:
         return None, None
-    capturing = torch.cuda.is_current_stream_capturing()
-    key = (w.data_ptr(), w._version, ks, str(w.device))
-    if not capturing:
-        hit = _PROJ_CACHE.get(key)
-        if hit is not None and (hit[1] is not None or not need_bwd):
-            _PROJ_CACHE.move_to_end(key)
-            torch.cuda.current_stream().wait_event(hit[2])
-            return hit[0], hit[1]
-    img_f = torch.empty(ks * 64 * 64 * 2, device=w.device, dtype=torch.float32)
-    img_b = torch.zeros((2 if ks > 4 else 1) * 2 * 2 * 256 * 32, device=w.device, dtype=torch.float32) if need_bwd else None
-    _lib.check(L.stmgcn_proj_pack_tc(w.data_ptr(), ks, img_f.data_ptr(), _p(img_b), _stream()), "proj_pack_tc")
-    if not capturing:
-        ev = torch.cuda.Event()
-        ev.record()
-        _PROJ_CACHE[key] = (img_f, img_b, ev, w)          # keeps `w` alive: a recycled data_ptr can never alias the key
-        while len(_PROJ_CACHE) > _W16_MAX:
-            _PROJ_CACHE.popitem(last=False)
-    return img_f, img_b
+
+    def pack():
+        img_f = torch.empty(ks * 64 * 64 * 2, device=w.device, dtype=torch.float32)
+        img_b = torch.zeros((2 if ks > 4 else 1) * 2 * 2 * 256 * 32, device=w.device, dtype=torch.float32) if need_bwd else None
+        _lib.check(L.stmgcn_proj_pack_tc(w.data_ptr(), ks, img_f.data_ptr(), _p(img_b), _stream()), "proj_pack_tc")
+        return dict(fwd=img_f, bwd=img_b)
+
+    img = _cached_images(_PROJ_IMAGES, [w], (ks,), pack, lambda hit: hit["bwd"] is not None or not need_bwd)
+    return img["fwd"], img["bwd"]
 
 
 def _proj_fwd(s: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], act: int, pool: Optional[torch.Tensor],
@@ -396,43 +412,24 @@ def set_lstm_planes(planes: int) -> None:
     _PLANES = planes
 
 
-_W16_CACHE: "OrderedDict" = OrderedDict()
-_W16_MAX = 24
-
-
 def _lstm16_images(weights: Sequence[torch.Tensor], n_layers: int, c_in: int):
-    """Operand images of the shared LSTM's parameters for the bf16-plane kernels (stmgcn_lstm16_pack), cached on
-    (storage, in-place version) of every parameter: re-packed only after an optimizer step changed them.  During CUDA
-    graph capture the cache is bypassed so the pack kernels become part of the graph (replays see updated weights)."""
-    capturing = torch.cuda.is_current_stream_capturing()
-    key = tuple((w.data_ptr(), w._version) for w in weights) + (c_in, str(weights[0].device))
-    if not capturing:
-        hit = _W16_CACHE.get(key)
-        if hit is not None:
-            _W16_CACHE.move_to_end(key)
-            torch.cuda.current_stream().wait_event(hit["event"])
-            return hit
-    dev = weights[0].device
-    wimg = [torch.empty(65536 if l == 0 else 131072, dtype=torch.uint8, device=dev) for l in range(n_layers)]
-    bias = [torch.empty(256, dtype=torch.float32, device=dev) for _ in range(n_layers)]
-    wih_t = torch.empty(c_in * 256, dtype=torch.float32, device=dev)
-    st = _stream()
-    for l in range(n_layers):
-        w_ih, w_hh, b_ih, b_hh = weights[4 * l:4 * l + 4]
-        _lib.check(L.stmgcn_lstm16_pack(w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), l, c_in,
-                                        wimg[l].data_ptr(), bias[l].data_ptr(), wih_t.data_ptr() if l == 0 else None, st),
-                   "lstm16_pack")
-    entry = dict(wimg=wimg, bias=bias, wih_t=wih_t, wimg_arr=_lib.ptr_array([v.data_ptr() for v in wimg]),
-                 bias_arr=_lib.ptr_array([v.data_ptr() for v in bias]),
-                 keep=list(weights))            # keeps the storages alive: a recycled data_ptr can never alias the key
-    if not capturing:
-        ev = torch.cuda.Event()
-        ev.record()
-        entry["event"] = ev
-        _W16_CACHE[key] = entry
-        while len(_W16_CACHE) > _W16_MAX:
-            _W16_CACHE.popitem(last=False)
-    return entry
+    """Operand images of the shared LSTM's parameters for the bf16-plane kernels (stmgcn_lstm16_pack)."""
+
+    def pack():
+        dev = weights[0].device
+        wimg = [torch.empty(65536 if l == 0 else 131072, dtype=torch.uint8, device=dev) for l in range(n_layers)]
+        bias = [torch.empty(256, dtype=torch.float32, device=dev) for _ in range(n_layers)]
+        wih_t = torch.empty(c_in * 256, dtype=torch.float32, device=dev)
+        st = _stream()
+        for l in range(n_layers):
+            w_ih, w_hh, b_ih, b_hh = weights[4 * l:4 * l + 4]
+            _lib.check(L.stmgcn_lstm16_pack(w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), l, c_in,
+                                            wimg[l].data_ptr(), bias[l].data_ptr(), wih_t.data_ptr() if l == 0 else None,
+                                            st), "lstm16_pack")
+        return dict(wimg=wimg, bias=bias, wih_t=wih_t, wimg_arr=_lib.ptr_array([v.data_ptr() for v in wimg]),
+                    bias_arr=_lib.ptr_array([v.data_ptr() for v in bias]))
+
+    return _cached_images(_LSTM16_IMAGES, weights, (c_in,), pack)
 
 
 def to_planes(x: torch.Tensor, planes: int) -> torch.Tensor:
@@ -495,7 +492,8 @@ def _lstm16_backward(xo, s_gate, tape, n_layers, planes, d_top):
     dev = xo.device
     rows_pad = ((rows + 127) // 128) * 128
     img = tape["img"]
-    torch.cuda.current_stream().wait_event(img["event"]) if "event" in img else None
+    if "event" in img:                 # a cached entry (no event: packed inside the CUDA graph being captured)
+        torch.cuda.current_stream().wait_event(img["event"])
     d_top_b = to_blocked(_f32c(d_top).view(rows, 64))
     dh_rec = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
     dc = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
