@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define STMGCN_ABI_VERSION 3
+#define STMGCN_ABI_VERSION 4
 
 /* error codes < 0 */
 #define STMGCN_ERR_ARG      (-1)   /* null pointer / bad enum */
@@ -91,18 +91,17 @@ int32_t stmgcn_obs_to_node_major(const float* obs, float* xo, float* xt, int64_t
                                  int64_t n, int64_t c, void* stream);
 
 /* ---- K2: stacked-K projection (GCN.py:37-42) --------------------------------------------------------
+ * Two kernel families, one set of entries each.  stmgcn_proj_fwd / _bwd run the exact-FFMA CUDA-core kernels for any
+ * shape, with pooling; stmgcn_proj_fwd_tc / _bwd_tc run the tcgen05 3xTF32 kernels (every fp32 operand split into tf32
+ * hi + lo, three passes) for p = q = 64 and ks <= 8, and reject anything else.
+ *
  * out[r,:] = act( sum_k S_k[r,:] W[k*p:(k+1)*p, :] + bias ),  r in [0, rows), S_k = s + k*stride_k
  * (rows x p, row-major), W: (ks*p, q) row-major, bias: q or NULL.
  * Optional gate pooling (STMGCN.py:41-42), requires q == p: pool[(r % b_inner)*q + j] +=
  * S_0[r,j] + out[r,j]  (caller zeroes pool; sum over regions of x_hat, not yet divided by N). */
 int32_t stmgcn_proj_fwd(const float* s, int64_t stride_k, int32_t ks, int64_t rows, int32_t p,
                         const float* w, const float* bias, int32_t q, int32_t act, float* out,
-                        float* pool, int64_t b_inner, const float* wimg, void* stream);
-/* Tensor-core operand images of W (ks*64, 64) for p = q = 64, ks <= 8 (3xTF32: every fp32 operand split into tf32 hi + lo, three tcgen05 passes):
- * img_fwd: ks*64*64*2 floats; img_bwd (may be NULL): one 2*2*256*32-float image per group of 4 supports (two images
- * when ks > 4), ZERO-FILLED by the caller (rows beyond ks*64 stay zero).  Passing wimg / wimg_t != NULL to stmgcn_proj_fwd / _bwd selects the tcgen05 kernels when
- * p = q = 64 (and, for the backward, a full d_out and u are given); otherwise the exact-FFMA kernels run. */
-int32_t stmgcn_proj_pack_tc(const float* w, int32_t ks, float* img_fwd, float* img_bwd, void* stream);
+                        float* pool, int64_t b_inner, void* stream);
 /* backward of the projection.  dZ = dOut (.) [out > 0] (act = RELU) with dOut either a full (rows, q)
  * tensor (d_out) or, when d_out_bcast != NULL, the broadcast dOut[r,:] = d_out_bcast[(r % b_inner), :] *
  * bcast_scale (the mean-pool adjoint dz/N, STMGCN.py:42).  dz_work: (rows, q) workspace receiving dZ.
@@ -111,8 +110,21 @@ int32_t stmgcn_proj_pack_tc(const float* w, int32_t ks, float* img_fwd, float* i
 int32_t stmgcn_proj_bwd(const float* s, int64_t stride_k, int32_t ks, int64_t rows, int32_t p,
                         const float* wt, int32_t q, int32_t act, const float* out, const float* d_out,
                         const float* d_out_bcast, float bcast_scale, int64_t b_inner, float* dz_work,
-                        float* dw, float* dbias, float* u, int64_t stride_u, const float* wimg_t,
-                        void* stream);
+                        float* dw, float* dbias, float* u, int64_t stride_u, void* stream);
+/* Tensor-core operand images of W (ks*64, 64), ks <= 8: img_fwd: ks*64*64*2 floats; img_bwd (may be NULL): one
+ * 2*2*256*32-float image per group of 4 supports (two images when ks > 4), ZERO-FILLED by the caller (rows beyond ks*64
+ * stay zero). */
+int32_t stmgcn_proj_pack_tc(const float* w, int32_t ks, float* img_fwd, float* img_bwd, void* stream);
+/* stmgcn_proj_fwd on the tensor cores: p = q = 64, 1 <= ks <= 8, no pooling; wimg = img_fwd of stmgcn_proj_pack_tc.
+ * s, wimg and out 16-byte aligned, stride_k a multiple of 4. */
+int32_t stmgcn_proj_fwd_tc(const float* s, int64_t stride_k, int32_t ks, int64_t rows, const float* wimg,
+                           const float* bias, int32_t act, float* out, void* stream);
+/* stmgcn_proj_bwd on the tensor cores: p = q = 64, 1 <= ks <= 8, a full d_out, and U is always produced (u required);
+ * wimg_t = img_bwd of stmgcn_proj_pack_tc.  s, wimg_t, out, d_out, dz_work and u 16-byte aligned, stride_k and stride_u
+ * multiples of 4. */
+int32_t stmgcn_proj_bwd_tc(const float* s, int64_t stride_k, int32_t ks, int64_t rows, const float* wimg_t,
+                           int32_t act, const float* out, const float* d_out, float* dz_work, float* dw, float* dbias,
+                           float* u, int64_t stride_u, void* stream);
 
 /* ---- K3a: context gate (STMGCN.py:42-43) -----------------------------------------------------------
  * z = pool / n_regions; a1 = z fcw^T + fcb; s = sigmoid(relu(a1) fcw^T + fcb).  All (B, T); fcw (T,T). */

@@ -5,18 +5,6 @@
 
 using namespace stmgcn;
 
-namespace stmgcn {
-bool proj_tc_applicable(int ks, int p, int q, const void* a, const void* b, const void* c);
-int32_t launch_proj_fwd_tc(const float* s, int64_t stride_k, int ks, int64_t rows, const float* wimg, const float* bias,
-                           int act, float* out, cudaStream_t st);
-int32_t launch_proj_bwd_tc(const float* d_out, const float* out_act, int act, int64_t rows, int ks, const float* wimg_t,
-                           float* dz_out, float* dbias, float* u, int64_t stride_u, cudaStream_t st);
-int32_t launch_pack_image(const float* src, int n_rows, int k_cols, int64_t rs, int64_t cs, float* img, int tile_rows,
-                          cudaStream_t st);
-int32_t launch_proj_tc_wgrad(const float* seg0, const float* seg1, const float* dz, int64_t rows, float* dw,
-                             cudaStream_t st);
-}
-
 namespace {
 
 struct ProjEpi {
@@ -171,32 +159,14 @@ int32_t launch_tall_auto(const ASegs& a, int64_t rows, int kd, const float* b, i
 
 extern "C" {
 
-int32_t stmgcn_proj_pack_tc(const float* w, int32_t ks, float* img_fwd, float* img_bwd, void* stream) {
-    STMGCN_REQUIRE(w && img_fwd, STMGCN_ERR_ARG, "proj_pack_tc: null pointer");
-    STMGCN_REQUIRE(ks >= 1 && ks <= 8, STMGCN_ERR_SHAPE, "proj_pack_tc: ks=%d (tensor-core path supports 1..8 supports)", ks);
-    cudaStream_t st = (cudaStream_t)stream;
-    // forward operand B[n = out col][k = ks*64 index] = W[k][n]
-    if (int32_t rc = launch_pack_image(w, 64, ks * 64, 1, 64, img_fwd, 64, st)) return rc;
-    // backward operand B[n = k*64+i][k' = out col] = W[n][k'], one 256-row image per group of 4 supports (caller
-    // zero-fills img_bwd: rows beyond the last support stay zero)
-    if (img_bwd) {
-        const int k0 = ks < 4 ? ks : 4;
-        if (int32_t rc = launch_pack_image(w, k0 * 64, 64, 64, 1, img_bwd, 256, st)) return rc;
-        if (ks > 4) return launch_pack_image(w + (int64_t)256 * 64, (ks - 4) * 64, 64, 64, 1, img_bwd + 2 * 2 * 256 * 32, 256, st);
-    }
-    return 0;
-}
-
 int32_t stmgcn_proj_fwd(const float* s, int64_t stride_k, int32_t ks, int64_t rows, int32_t p, const float* w,
                         const float* bias, int32_t q, int32_t act, float* out, float* pool, int64_t b_inner,
-                        const float* wimg, void* stream) {
+                        void* stream) {
     STMGCN_REQUIRE(s && w && out, STMGCN_ERR_ARG, "proj_fwd: null pointer");
     STMGCN_REQUIRE(ks >= 1 && ks <= kMaxSegs, STMGCN_ERR_SHAPE, "proj_fwd: %d supports (max %d)", ks, kMaxSegs);
     STMGCN_REQUIRE(rows > 0 && p > 0 && q > 0, STMGCN_ERR_SHAPE, "proj_fwd: bad shape");
     STMGCN_REQUIRE(act == STMGCN_ACT_NONE || act == STMGCN_ACT_RELU, STMGCN_ERR_ARG, "proj_fwd: act=%d", act);
     cudaStream_t st = (cudaStream_t)stream;
-    if (wimg && !pool && proj_tc_applicable(ks, p, q, s, out, nullptr) && stride_k % 4 == 0)   // tcgen05 path (proj_tc.cu)
-        return launch_proj_fwd_tc(s, stride_k, ks, rows, wimg, bias, act, out, st);
     ASegs a{};
     a.nseg = ks;
     a.segw = p;
@@ -227,7 +197,7 @@ int32_t stmgcn_proj_fwd(const float* s, int64_t stride_k, int32_t ks, int64_t ro
 int32_t stmgcn_proj_bwd(const float* s, int64_t stride_k, int32_t ks, int64_t rows, int32_t p, const float* wt,
                         int32_t q, int32_t act, const float* out, const float* d_out, const float* d_out_bcast,
                         float bcast_scale, int64_t b_inner, float* dz_work, float* dw, float* dbias, float* u,
-                        int64_t stride_u, const float* wimg_t, void* stream) {
+                        int64_t stride_u, void* stream) {
     STMGCN_REQUIRE(s && out && dz_work && dw, STMGCN_ERR_ARG, "proj_bwd: null pointer");
     STMGCN_REQUIRE((d_out != nullptr) != (d_out_bcast != nullptr), STMGCN_ERR_ARG,
                    "proj_bwd: exactly one of d_out / d_out_bcast");
@@ -236,23 +206,6 @@ int32_t stmgcn_proj_bwd(const float* s, int64_t stride_k, int32_t ks, int64_t ro
     STMGCN_REQUIRE(!d_out_bcast || (b_inner > 0 && rows % b_inner == 0), STMGCN_ERR_SHAPE, "proj_bwd: b_inner");
     STMGCN_REQUIRE(!u || wt, STMGCN_ERR_ARG, "proj_bwd: u requested without wt");
     cudaStream_t st = (cudaStream_t)stream;
-    if (wimg_t && u && d_out && proj_tc_applicable(ks, p, q, s, out, d_out) && aligned16(dz_work) && aligned16(u) &&
-        stride_k % 4 == 0 && stride_u % 4 == 0) {
-        // tcgen05 path (proj_tc.cu): dZ + bias gradient + U in one kernel, then dW per 128-row block of W
-        // U has 64*ks columns; one launch produces up to 256 of them (supports 0..3), a second one the rest (it re-forms
-        // dZ in its loader but neither stores it nor accumulates the bias gradient again)
-        if (int32_t rc = launch_proj_bwd_tc(d_out, out, act, rows, ks < 4 ? ks : 4, wimg_t, dz_work, dbias, u, stride_u, st)) return rc;
-        if (ks > 4)
-            if (int32_t rc = launch_proj_bwd_tc(d_out, out, act, rows, ks - 4, wimg_t + 2 * 2 * 256 * 32, nullptr, nullptr,
-                                                u + 4 * stride_u, stride_u, st))
-                return rc;
-        for (int k0 = 0; k0 < ks; k0 += 2) {
-            const float* s0 = s + (int64_t)k0 * stride_k;
-            const float* s1 = k0 + 1 < ks ? s0 + stride_k : nullptr;     // nullptr: the 64-row tail block of W
-            if (int32_t rc = launch_proj_tc_wgrad(s0, s1, dz_work, rows, dw + (int64_t)k0 * 64 * 64, st)) return rc;
-        }
-        return 0;
-    }
     {
         const int64_t total = rows * q;
         int64_t blocks = ceil_div(total, 256 * 8);

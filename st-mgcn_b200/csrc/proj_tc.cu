@@ -533,14 +533,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) proj_tc_wgrad_kernel(const __gr
     if (warp == kMmaWarp) tmem_dealloc(tmem_base, kWgN);
 }
 
-}  // namespace
-
-namespace stmgcn {
-
-bool proj_tc_applicable(int ks, int p, int q, const void* a, const void* b, const void* c) {
-    return p == 64 && q == 64 && ks >= 1 && ks <= 8 && aligned16(a) && aligned16(b) && (!c || aligned16(c));
-}
-
+// ---- host launchers ----------------------------------------------------------------------------------------
 // forward: out = act(sum_k S_k W_k + bias); wimg = image of B[n][k] = W[k][n] (2*ks k-blocks of [hi|lo] [64][32])
 int32_t launch_proj_fwd_tc(const float* s, int64_t stride_k, int ks, int64_t rows, const float* wimg, const float* bias,
                            int act, float* out, cudaStream_t st) {
@@ -612,4 +605,63 @@ int32_t launch_pack_image(const float* src, int n_rows, int k_cols, int64_t rs, 
     return check_launch("pack_image");
 }
 
-}  // namespace stmgcn
+}  // namespace
+
+extern "C" {
+
+int32_t stmgcn_proj_pack_tc(const float* w, int32_t ks, float* img_fwd, float* img_bwd, void* stream) {
+    STMGCN_REQUIRE(w && img_fwd, STMGCN_ERR_ARG, "proj_pack_tc: null pointer");
+    STMGCN_REQUIRE(ks >= 1 && ks <= 8, STMGCN_ERR_SHAPE, "proj_pack_tc: ks=%d (tensor-core path supports 1..8 supports)", ks);
+    cudaStream_t st = (cudaStream_t)stream;
+    // forward operand B[n = out col][k = ks*64 index] = W[k][n]
+    if (int32_t rc = launch_pack_image(w, 64, ks * 64, 1, 64, img_fwd, 64, st)) return rc;
+    // backward operand B[n = k*64+i][k' = out col] = W[n][k'], one 256-row image per group of 4 supports (caller
+    // zero-fills img_bwd: rows beyond the last support stay zero)
+    if (img_bwd) {
+        const int k0 = ks < 4 ? ks : 4;
+        if (int32_t rc = launch_pack_image(w, k0 * 64, 64, 64, 1, img_bwd, 256, st)) return rc;
+        if (ks > 4) return launch_pack_image(w + (int64_t)256 * 64, (ks - 4) * 64, 64, 64, 1, img_bwd + 2 * 2 * 256 * 32, 256, st);
+    }
+    return 0;
+}
+
+int32_t stmgcn_proj_fwd_tc(const float* s, int64_t stride_k, int32_t ks, int64_t rows, const float* wimg,
+                           const float* bias, int32_t act, float* out, void* stream) {
+    STMGCN_REQUIRE(s && wimg && out, STMGCN_ERR_ARG, "proj_fwd_tc: null pointer");
+    STMGCN_REQUIRE(act == STMGCN_ACT_NONE || act == STMGCN_ACT_RELU, STMGCN_ERR_ARG, "proj_fwd_tc: act=%d", act);
+    STMGCN_REQUIRE(ks >= 1 && ks <= 8 && rows > 0, STMGCN_ERR_SHAPE, "proj_fwd_tc: ks=%d rows=%lld (1..8 supports)", ks,
+                   (long long)rows);
+    STMGCN_REQUIRE(aligned16(s) && aligned16(wimg) && aligned16(out) && stride_k % 4 == 0, STMGCN_ERR_ALIGN,
+                   "proj_fwd_tc: s, wimg and out must be 16-byte aligned and stride_k a multiple of 4");
+    return launch_proj_fwd_tc(s, stride_k, ks, rows, wimg, bias, act, out, (cudaStream_t)stream);
+}
+
+int32_t stmgcn_proj_bwd_tc(const float* s, int64_t stride_k, int32_t ks, int64_t rows, const float* wimg_t, int32_t act,
+                           const float* out, const float* d_out, float* dz_work, float* dw, float* dbias, float* u,
+                           int64_t stride_u, void* stream) {
+    STMGCN_REQUIRE(s && wimg_t && out && d_out && dz_work && dw && u, STMGCN_ERR_ARG, "proj_bwd_tc: null pointer");
+    STMGCN_REQUIRE(act == STMGCN_ACT_NONE || act == STMGCN_ACT_RELU, STMGCN_ERR_ARG, "proj_bwd_tc: act=%d", act);
+    STMGCN_REQUIRE(ks >= 1 && ks <= 8 && rows > 0, STMGCN_ERR_SHAPE, "proj_bwd_tc: ks=%d rows=%lld (1..8 supports)", ks,
+                   (long long)rows);
+    STMGCN_REQUIRE(aligned16(s) && aligned16(wimg_t) && aligned16(out) && aligned16(d_out) && aligned16(dz_work) &&
+                       aligned16(u) && stride_k % 4 == 0 && stride_u % 4 == 0,
+                   STMGCN_ERR_ALIGN, "proj_bwd_tc: s, wimg_t, out, d_out, dz_work and u must be 16-byte aligned, "
+                   "stride_k and stride_u multiples of 4");
+    cudaStream_t st = (cudaStream_t)stream;
+    // dZ + bias gradient + U in one kernel.  U has 64*ks columns; one launch produces up to 256 of them (supports 0..3), a
+    // second one the rest (it re-forms dZ in its loader but neither stores it nor accumulates the bias gradient again)
+    if (int32_t rc = launch_proj_bwd_tc(d_out, out, act, rows, ks < 4 ? ks : 4, wimg_t, dz_work, dbias, u, stride_u, st)) return rc;
+    if (ks > 4)
+        if (int32_t rc = launch_proj_bwd_tc(d_out, out, act, rows, ks - 4, wimg_t + 2 * 2 * 256 * 32, nullptr, nullptr,
+                                            u + 4 * stride_u, stride_u, st))
+            return rc;
+    // dW per 128-row block of W
+    for (int k0 = 0; k0 < ks; k0 += 2) {
+        const float* s0 = s + (int64_t)k0 * stride_k;
+        const float* s1 = k0 + 1 < ks ? s0 + stride_k : nullptr;     // nullptr: the 64-row tail block of W
+        if (int32_t rc = launch_proj_tc_wgrad(s0, s1, dz_work, rows, dw + (int64_t)k0 * 64 * 64, st)) return rc;
+    }
+    return 0;
+}
+
+}  // extern "C"

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STMGCN_LIB_PATH") or os.path.join(os.path.dirname(_HERE), "lib", "libstmgcn_b200.so")
 
 ACT_NONE, ACT_RELU = 0, 1
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 # (name, restype, argtypes) -- one row per symbol in include/stmgcn_b200.h
 _P = c_void_p
@@ -33,10 +33,13 @@ SIGNATURES = [
     ("stmgcn_to_bf16", c_int32, [_P, _P, c_int64, _P]),
     ("stmgcn_obs_to_node_major", c_int32, [_P, _P, _P, c_int64, c_int64, c_int64, c_int64, _P]),
     ("stmgcn_proj_fwd", c_int32, [_P, c_int64, c_int32, c_int64, c_int32, _P, _P, c_int32, c_int32, _P, _P,
-                                  c_int64, _P, _P]),
-    ("stmgcn_proj_pack_tc", c_int32, [_P, c_int32, _P, _P, _P]),
+                                  c_int64, _P]),
     ("stmgcn_proj_bwd", c_int32, [_P, c_int64, c_int32, c_int64, c_int32, _P, c_int32, c_int32, _P, _P, _P,
-                                  c_float, c_int64, _P, _P, _P, _P, c_int64, _P, _P]),
+                                  c_float, c_int64, _P, _P, _P, _P, c_int64, _P]),
+    ("stmgcn_proj_pack_tc", c_int32, [_P, c_int32, _P, _P, _P]),
+    ("stmgcn_proj_fwd_tc", c_int32, [_P, c_int64, c_int32, c_int64, _P, _P, c_int32, _P, _P]),
+    ("stmgcn_proj_bwd_tc", c_int32, [_P, c_int64, c_int32, c_int64, _P, c_int32, _P, _P, _P, _P, _P, _P, c_int64,
+                                     _P]),
     ("stmgcn_gate_fwd", c_int32, [_P, c_int64, c_int32, c_int64, _P, _P, _P, _P, _P, _P]),
     ("stmgcn_gate_bwd", c_int32, [_P, _P, _P, _P, c_int64, c_int32, _P, _P, _P, _P, _P]),
     ("stmgcn_lstm_step_fwd", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, c_int32, c_int64, _P, _P,

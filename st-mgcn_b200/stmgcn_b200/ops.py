@@ -9,7 +9,7 @@ Functions (reference lines they replace):
   ChebGCN          GCN.py:24-43 on a sparse L~ (recurrence on features) -> out (N,B,q)
   TemporalPool     STMGCN.py:40-42: GCN over time-as-features + residual + sum over regions -> (B,T)
   ContextGate      STMGCN.py:42-43: /N, fc, relu, fc (same weights), sigmoid -> s (B,T)
-  SharedLSTM       STMGCN.py:44,47-50: modulate + 3-layer shared LSTM, one library call per timestep (lstm16.cu / lstm.cu)
+  SharedLSTM       STMGCN.py:44,47-50: modulate + 3-layer shared LSTM -> SharedLSTM16 (lstm16.cu) or SharedLSTMExact (lstm.cu)
   FuseOut          STMGCN.py:116-118: sum over graphs + output FC -> (B,N,C)
 """
 from __future__ import annotations
@@ -191,11 +191,19 @@ def _cached_images(store: "OrderedDict", params: Sequence[torch.Tensor], extra: 
     return entry
 
 
-def _proj_images(w: torch.Tensor, ks: int, p: int, need_bwd: bool):
-    """tcgen05 operand images (forward, backward) of the projection weights (p = q = 64, ks <= 8), or (None, None).
-    The backward image is packed only when ``need_bwd``; an entry without it is re-packed when a later call needs it."""
-    if lstm_path() != "tc" or p != 64 or w.shape[1] != 64 or ks > 8:
-        return None, None
+def _proj_tc(ks: int, p: int, q: int) -> bool:
+    """Whether ChebGCN's projection runs on the tcgen05 3xTF32 entries (stmgcn_proj_fwd_tc / _bwd_tc) rather than the
+    exact-FFMA ones.  Those entries also require 16-byte aligned pointers and strides that are multiples of 4 floats;
+    everything ChebGCN passes them is allocated here (build_stack, torch.empty; stride_k = N*B*64), so that holds by
+    construction, except for the incoming gradient d_out.  ChebGCN.backward therefore takes the tensor-core entry only
+    when the forward took it (it packed the backward image), dX is needed (the entry always produces U) and d_out is
+    16-byte aligned; otherwise it calls the FFMA entry."""
+    return lstm_path() == "tc" and p == 64 and q == 64 and ks <= 8
+
+
+def _proj_images(w: torch.Tensor, ks: int, need_bwd: bool):
+    """tcgen05 operand images (forward, backward) of the projection weights (64, 64 per support, ks <= 8).  The backward
+    image is packed only when ``need_bwd``; an entry without it is re-packed when a later call needs it."""
 
     def pack():
         img_f = torch.empty(ks * 64 * 64 * 2, device=w.device, dtype=torch.float32)
@@ -208,18 +216,25 @@ def _proj_images(w: torch.Tensor, ks: int, p: int, need_bwd: bool):
 
 
 def _proj_fwd(s: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], act: int, pool: Optional[torch.Tensor],
-              b_inner: int, wimg: Optional[torch.Tensor] = None) -> torch.Tensor:
+              b_inner: int) -> torch.Tensor:
     ks, n, b, p = s.shape
     q = w.shape[1]
     out = torch.empty((n, b, q), device=s.device, dtype=torch.float32)
     _lib.check(L.stmgcn_proj_fwd(s.data_ptr(), n * b * p, ks, n * b, p, w.data_ptr(), _p(bias), q, act,
-                                 out.data_ptr(), _p(pool), b_inner, _p(wimg), _stream()), "proj_fwd")
+                                 out.data_ptr(), _p(pool), b_inner, _stream()), "proj_fwd")
+    return out
+
+
+def _proj_fwd_tc(s: torch.Tensor, wimg: torch.Tensor, bias: Optional[torch.Tensor], act: int) -> torch.Tensor:
+    ks, n, b, _ = s.shape
+    out = torch.empty((n, b, 64), device=s.device, dtype=torch.float32)
+    _lib.check(L.stmgcn_proj_fwd_tc(s.data_ptr(), n * b * 64, ks, n * b, wimg.data_ptr(), _p(bias), act, out.data_ptr(),
+                                    _stream()), "proj_fwd_tc")
     return out
 
 
 def _proj_bwd(s: torch.Tensor, w: torch.Tensor, act: int, out: torch.Tensor, d_out: Optional[torch.Tensor],
-              d_bcast: Optional[torch.Tensor], scale: float, b_inner: int, need_bias: bool, need_u: bool,
-              wimg_t: Optional[torch.Tensor] = None):
+              d_bcast: Optional[torch.Tensor], scale: float, b_inner: int, need_bias: bool, need_u: bool):
     ks, n, b, p = s.shape
     q = w.shape[1]
     dw = torch.zeros_like(w, dtype=torch.float32)
@@ -229,7 +244,20 @@ def _proj_bwd(s: torch.Tensor, w: torch.Tensor, act: int, out: torch.Tensor, d_o
     wt = w.t().contiguous() if need_u else None
     _lib.check(L.stmgcn_proj_bwd(s.data_ptr(), n * b * p, ks, n * b, p, _p(wt), q, act, out.data_ptr(), _p(d_out),
                                  _p(d_bcast), scale, b_inner, dz.data_ptr(), dw.data_ptr(), _p(db), _p(u),
-                                 n * b * p, _p(wimg_t), _stream()), "proj_bwd")
+                                 n * b * p, _stream()), "proj_bwd")
+    return dw, db, u
+
+
+def _proj_bwd_tc(s: torch.Tensor, w: torch.Tensor, wimg_t: torch.Tensor, act: int, out: torch.Tensor,
+                 d_out: torch.Tensor, need_bias: bool):
+    ks, n, b, _ = s.shape
+    dw = torch.zeros_like(w, dtype=torch.float32)
+    db = torch.zeros(64, device=s.device, dtype=torch.float32) if need_bias else None
+    dz = torch.empty((n * b, 64), device=s.device, dtype=torch.float32)
+    u = torch.empty_like(s)
+    _lib.check(L.stmgcn_proj_bwd_tc(s.data_ptr(), n * b * 64, ks, n * b, wimg_t.data_ptr(), act, out.data_ptr(),
+                                    d_out.data_ptr(), dz.data_ptr(), dw.data_ptr(), _p(db), u.data_ptr(), n * b * 64,
+                                    _stream()), "proj_bwd_tc")
     return dw, db, u
 
 
@@ -264,8 +292,12 @@ class ChebGCN(torch.autograd.Function):
         # moved by 2-3.6e-2 on the golden case (measured), past that mode's 2e-2 bar -- and its F = B*T rows are cheap.
         s = build_stack(sset, x, gather16=True)
         need_grad = any(ctx.needs_input_grad)
-        img_f, img_b = _proj_images(w, sset.ks, x.shape[2], need_grad)
-        out = _proj_fwd(s, w, bias_c, act, None, x.shape[1], img_f)
+        img_b = None
+        if _proj_tc(sset.ks, x.shape[2], w.shape[1]):
+            img_f, img_b = _proj_images(w, sset.ks, need_grad)
+            out = _proj_fwd_tc(s, img_f, bias_c, act)
+        else:
+            out = _proj_fwd(s, w, bias_c, act, None, x.shape[1])
         ctx.sset, ctx.act, ctx.has_bias = sset, act, bias is not None
         if need_grad:
             ctx.save_for_backward(s, w, out, img_b)
@@ -276,7 +308,10 @@ class ChebGCN(torch.autograd.Function):
         s, w, out, img_b = ctx.saved_tensors
         need_dx = ctx.needs_input_grad[0]
         d_out = _f32c(d_out)
-        dw, db, u = _proj_bwd(s, w, ctx.act, out, d_out, None, 1.0, s.shape[2], ctx.has_bias, need_dx, img_b)
+        if img_b is not None and need_dx and d_out.data_ptr() % 16 == 0:      # see _proj_tc
+            dw, db, u = _proj_bwd_tc(s, w, img_b, ctx.act, out, d_out, ctx.has_bias)
+        else:
+            dw, db, u = _proj_bwd(s, w, ctx.act, out, d_out, None, 1.0, s.shape[2], ctx.has_bias, need_dx)
         dx = adjoint_stack_(ctx.sset, u) if need_dx else None
         return dx, dw, db, None, None
 
@@ -441,37 +476,6 @@ def to_planes(x: torch.Tensor, planes: int) -> torch.Tensor:
     return torch.stack([hi, lo], dim=-3).contiguous()
 
 
-def _lstm16_forward(xo, s_gate, h0c, c0c, n_layers, want_state, weights, planes, keep_tape):
-    """Forward of the bf16-plane path.  Returns (h_top (N,B,64), h_n, c_n, tape dict or None)."""
-    n, b, t_len, c_in = xo.shape
-    rows = n * b
-    dev = xo.device
-    rows_pad = ((rows + 127) // 128) * 128
-    img = _lstm16_images(weights, n_layers, c_in)
-    hp = torch.empty((n_layers, t_len, planes, rows, 64), device=dev, dtype=torch.bfloat16)
-    cs = torch.empty((n_layers, t_len, rows_pad, 64), device=dev, dtype=torch.float32)
-    h0p = to_planes(h0c, planes) if h0c is not None else None        # (L, P, R, 64)
-    c0b = to_blocked(c0c) if c0c is not None else None
-    if want_state:
-        h_n = torch.empty((n_layers, rows, 64), device=dev, dtype=torch.float32)
-        h_top = h_n[n_layers - 1]
-    else:
-        h_n = None
-        h_top = torch.empty((rows, 64), device=dev, dtype=torch.float32)
-    st = _stream()
-    for t in range(t_len):
-        _lib.check(L.stmgcn_lstm16_step_fwd(t, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
-                                            img["wimg_arr"], img["bias_arr"], img["wih_t"].data_ptr(), _p(h0p), _p(c0b),
-                                            hp.data_ptr(), cs.data_ptr(), h_top.data_ptr(), _p(h_n), st),
-                   "lstm16_step_fwd")
-    if want_state:
-        c_n = from_blocked(cs[:, t_len - 1], rows)
-    else:
-        h_n = c_n = torch.empty(0, device=dev, dtype=torch.float32)
-    tape = dict(hp=hp, cs=cs, h0p=h0p, c0b=c0b, img=img) if keep_tape else None
-    return h_top.view(n, b, 64), h_n, c_n, tape
-
-
 _ZERO_TILES: dict = {}
 
 
@@ -483,87 +487,111 @@ def _zero_tile(dev: torch.device) -> torch.Tensor:
     return _ZERO_TILES[key]
 
 
-def _lstm16_backward(xo, s_gate, tape, n_layers, planes, d_top):
-    """BPTT of the bf16-plane path: ONE fused launch per layer over all timesteps (gate recompute + pointwise + data
-    gradient + weight gradient, stmgcn_lstm16_layer_bwd), layers top-down, then one reduction per layer.
-    Returns (d_s, [native nn.LSTM gradients])."""
-    n, b, t_len, c_in = xo.shape
-    rows = n * b
-    dev = xo.device
-    rows_pad = ((rows + 127) // 128) * 128
-    img = tape["img"]
-    if "event" in img:                 # a cached entry (no event: packed inside the CUDA graph being captured)
-        torch.cuda.current_stream().wait_event(img["event"])
-    d_top_b = to_blocked(_f32c(d_top).view(rows, 64))
-    dh_rec = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
-    dc = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
-    # dx of a layer for every timestep: written by layer l, read by layer l - 1 (two buffers ping-pong down the stack)
-    dx_bufs = [torch.empty((t_len, rows_pad, 64), device=dev, dtype=torch.float32) for _ in range(min(2, n_layers - 1))]
-    d_s = torch.zeros((b, t_len), device=dev, dtype=torch.float32)
-    dbp = torch.zeros((n_layers, 256), device=dev, dtype=torch.float32)
-    grid = int(L.stmgcn_lstm16_grid(rows))
-    scratch = torch.empty((n_layers, grid, 128 * 256), device=dev, dtype=torch.float32)
-    zero = _zero_tile(dev)
-    st = _stream()
-    dh_in = d_top_b
-    for l in range(n_layers - 1, -1, -1):
-        dx_out = dx_bufs[(n_layers - 1 - l) % 2] if l > 0 else None
-        _lib.check(L.stmgcn_lstm16_layer_bwd(l, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
-                                             img["wimg"][l].data_ptr(), img["bias"][l].data_ptr(), img["wih_t"].data_ptr(),
-                                             _p(tape["h0p"]), _p(tape["c0b"]), tape["hp"].data_ptr(), tape["cs"].data_ptr(),
-                                             dh_in.data_ptr(), _p(dx_out), dh_rec.data_ptr(), dc.data_ptr(), d_s.data_ptr(),
-                                             dbp[l].data_ptr(), scratch[l].data_ptr(), zero.data_ptr(), st), "lstm16_layer_bwd")
-        dh_in = dx_out
-    grads = []
-    for l in range(n_layers):
-        in_l = c_in if l == 0 else 64
-        d_w_ih = torch.empty((256, in_l), device=dev, dtype=torch.float32)
-        d_w_hh = torch.empty((256, 64), device=dev, dtype=torch.float32)
-        d_b_ih = torch.empty(256, device=dev, dtype=torch.float32)
-        d_b_hh = torch.empty(256, device=dev, dtype=torch.float32)
-        _lib.check(L.stmgcn_lstm16_wgrad_reduce(l, c_in, grid, scratch[l].data_ptr(), dbp[l].data_ptr(), d_w_ih.data_ptr(),
-                                                d_w_hh.data_ptr(), d_b_ih.data_ptr(), d_b_hh.data_ptr(), st),
-                   "lstm16_wgrad_reduce")
-        grads += [d_w_ih, d_w_hh, d_b_ih, d_b_hh]
-    return d_s, grads
+def _lstm_inputs(xo, s_gate, h0, c0, weights):
+    """The shared LSTM's inputs as the kernels of both families read them: CUDA, fp32, contiguous."""
+    _require_cuda(xo, s_gate, *weights)
+    return (_f32c(xo), _f32c(s_gate), _f32c(h0) if h0 is not None else None, _f32c(c0) if c0 is not None else None,
+            [_f32c(w) for w in weights])
 
 
-class SharedLSTM(torch.autograd.Function):
-    """h_top (N,B,H) of the shared multi-layer LSTM over rows r = n*B + b; input ``xo * s[b,t]``.
-
-    forward(xo (N,B,T,C), s (B,T), h0|None, c0|None (L,R,H), n_layers, hid, want_state, *lstm_weights) where
-    lstm_weights = [w_ih_l0, w_hh_l0, b_ih_l0, b_hh_l0, w_ih_l1, ...] (nn.LSTM names/shapes).
-    Returns (h_top, h_n (L,R,H), c_n (L,R,H)); the last two are not differentiable.
-
-    Two kernel families (include/stmgcn_b200.h):
-    * H = 64, C <= 4, T <= 64 (the reference's configuration, Main.py:62) and ``lstm_path() == "tc"``: the tcgen05 bf16-plane
-      kernels of lstm16.cu -- tape = hidden-state planes + cell state, no gate tape, fused recompute backward;
-    * anything else, or ``lstm_path() == "fma"``: the exact-fp32 CUDA-core kernels of lstm.cu with their own tape
-      (hs, cs, gates); their backward overwrites the gate tape in place, so it can run only once per forward.
-    """
+class SharedLSTM16(torch.autograd.Function):
+    """:class:`SharedLSTM` on the tcgen05 bf16-plane kernels of lstm16.cu (H = 64, C <= 4, T <= 64).  Tape: the hidden
+    states as bf16 planes plus the cell state, no gate tape.  The backward recomputes the gates: ONE fused launch per
+    layer over all timesteps (gate recompute + pointwise + data gradient + weight gradient, stmgcn_lstm16_layer_bwd),
+    layers top-down, then one reduction per layer."""
 
     @staticmethod
     def forward(ctx, xo, s_gate, h0, c0, n_layers: int, hid: int, want_state: bool, *weights):
-        _require_cuda(xo, s_gate, *weights)
-        xo, s_gate = _f32c(xo), _f32c(s_gate)
-        weights = [_f32c(w) for w in weights]
+        xo, s_gate, h0, c0, weights = _lstm_inputs(xo, s_gate, h0, c0, weights)
         n, b, t_len, c_in = xo.shape
         rows = n * b
         dev = xo.device
-        h0c = _f32c(h0) if h0 is not None else None
-        c0c = _f32c(c0) if c0 is not None else None
+        rows_pad = ((rows + 127) // 128) * 128
+        planes = lstm_planes()
+        img = _lstm16_images(weights, n_layers, c_in)
+        hp = torch.empty((n_layers, t_len, planes, rows, 64), device=dev, dtype=torch.bfloat16)
+        cs = torch.empty((n_layers, t_len, rows_pad, 64), device=dev, dtype=torch.float32)
+        h0p = to_planes(h0, planes) if h0 is not None else None        # (L, P, R, 64)
+        c0b = to_blocked(c0) if c0 is not None else None
+        if want_state:
+            h_n = torch.empty((n_layers, rows, 64), device=dev, dtype=torch.float32)
+            h_top = h_n[n_layers - 1]
+        else:
+            h_n = None
+            h_top = torch.empty((rows, 64), device=dev, dtype=torch.float32)
+        st = _stream()
+        for t in range(t_len):
+            _lib.check(L.stmgcn_lstm16_step_fwd(t, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
+                                                img["wimg_arr"], img["bias_arr"], img["wih_t"].data_ptr(), _p(h0p), _p(c0b),
+                                                hp.data_ptr(), cs.data_ptr(), h_top.data_ptr(), _p(h_n), st),
+                       "lstm16_step_fwd")
+        if want_state:
+            c_n = from_blocked(cs[:, t_len - 1], rows)
+        else:
+            h_n = c_n = torch.empty(0, device=dev, dtype=torch.float32)
+        ctx.mark_non_differentiable(h_n, c_n)
+        if any(ctx.needs_input_grad):
+            ctx.n_layers, ctx.planes = n_layers, planes
+            ctx.tape = dict(hp=hp, cs=cs, h0p=h0p, c0b=c0b, img=img)
+            ctx.save_for_backward(xo, s_gate)
+        return h_top.view(n, b, 64), h_n, c_n
+
+    @staticmethod
+    def backward(ctx, d_top, _dhn, _dcn):
+        xo, s_gate = ctx.saved_tensors
+        tape, n_layers, planes = ctx.tape, ctx.n_layers, ctx.planes
+        n, b, t_len, c_in = xo.shape
+        rows = n * b
+        dev = xo.device
+        rows_pad = ((rows + 127) // 128) * 128
+        img = tape["img"]
+        if "event" in img:                 # a cached entry (no event: packed inside the CUDA graph being captured)
+            torch.cuda.current_stream().wait_event(img["event"])
+        d_top_b = to_blocked(_f32c(d_top).view(rows, 64))
+        dh_rec = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
+        dc = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
+        # dx of a layer for every timestep: written by layer l, read by layer l - 1 (two buffers ping-pong down the stack)
+        dx_bufs = [torch.empty((t_len, rows_pad, 64), device=dev, dtype=torch.float32) for _ in range(min(2, n_layers - 1))]
+        d_s = torch.zeros((b, t_len), device=dev, dtype=torch.float32)
+        dbp = torch.zeros((n_layers, 256), device=dev, dtype=torch.float32)
+        grid = int(L.stmgcn_lstm16_grid(rows))
+        scratch = torch.empty((n_layers, grid, 128 * 256), device=dev, dtype=torch.float32)
+        zero = _zero_tile(dev)
+        st = _stream()
+        dh_in = d_top_b
+        for l in range(n_layers - 1, -1, -1):
+            dx_out = dx_bufs[(n_layers - 1 - l) % 2] if l > 0 else None
+            _lib.check(L.stmgcn_lstm16_layer_bwd(l, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
+                                                 img["wimg"][l].data_ptr(), img["bias"][l].data_ptr(), img["wih_t"].data_ptr(),
+                                                 _p(tape["h0p"]), _p(tape["c0b"]), tape["hp"].data_ptr(), tape["cs"].data_ptr(),
+                                                 dh_in.data_ptr(), _p(dx_out), dh_rec.data_ptr(), dc.data_ptr(), d_s.data_ptr(),
+                                                 dbp[l].data_ptr(), scratch[l].data_ptr(), zero.data_ptr(), st), "lstm16_layer_bwd")
+            dh_in = dx_out
+        w_grads = []
+        for l in range(n_layers):
+            in_l = c_in if l == 0 else 64
+            d_w_ih = torch.empty((256, in_l), device=dev, dtype=torch.float32)
+            d_w_hh = torch.empty((256, 64), device=dev, dtype=torch.float32)
+            d_b_ih = torch.empty(256, device=dev, dtype=torch.float32)
+            d_b_hh = torch.empty(256, device=dev, dtype=torch.float32)
+            _lib.check(L.stmgcn_lstm16_wgrad_reduce(l, c_in, grid, scratch[l].data_ptr(), dbp[l].data_ptr(), d_w_ih.data_ptr(),
+                                                    d_w_hh.data_ptr(), d_b_ih.data_ptr(), d_b_hh.data_ptr(), st),
+                       "lstm16_wgrad_reduce")
+            w_grads += [d_w_ih, d_w_hh, d_b_ih, d_b_hh]
+        return (None, d_s, None, None, None, None, None, *w_grads)
+
+
+class SharedLSTMExact(torch.autograd.Function):
+    """:class:`SharedLSTM` on the exact-fp32 CUDA-core kernels of lstm.cu (any H <= 128).  Tape: hs, cs and the
+    post-activation gates; the backward overwrites the gate tape in place, so it can run only once per forward."""
+
+    @staticmethod
+    def forward(ctx, xo, s_gate, h0, c0, n_layers: int, hid: int, want_state: bool, *weights):
+        xo, s_gate, h0, c0, weights = _lstm_inputs(xo, s_gate, h0, c0, weights)
+        n, b, t_len, c_in = xo.shape
+        rows = n * b
+        dev = xo.device
         need_grad = any(ctx.needs_input_grad)
-        ctx.dims = (n, b, t_len, c_in, n_layers, hid)
-        if hid == 64 and lstm_path() == "tc" and c_in <= 4 and t_len <= 64:
-            planes = lstm_planes()
-            h_top, h_n, c_n, tape = _lstm16_forward(xo, s_gate, h0c, c0c, n_layers, want_state, weights, planes, need_grad)
-            ctx.mark_non_differentiable(h_n, c_n)
-            ctx.planes16 = True
-            if need_grad:
-                ctx.tape16, ctx.planes = tape, planes
-                ctx.save_for_backward(xo, s_gate)
-            return h_top, h_n, c_n
-        ctx.planes16 = False
         wx, wp, bp, wpt = _pack_lstm(weights, n_layers, hid)
         hs = torch.empty((n_layers, t_len, rows, hid), device=dev, dtype=torch.float32)
         cs = torch.empty((n_layers, t_len, rows, hid), device=dev, dtype=torch.float32)
@@ -572,10 +600,11 @@ class SharedLSTM(torch.autograd.Function):
         st = _stream()
         for t in range(t_len):
             _lib.check(L.stmgcn_lstm_step_fwd(t, t_len, n_layers, rows, hid, c_in, b, xo.data_ptr(),
-                                              s_gate.data_ptr(), wx.data_ptr(), wp_arr, bp_arr, _p(h0c), _p(c0c),
+                                              s_gate.data_ptr(), wx.data_ptr(), wp_arr, bp_arr, _p(h0), _p(c0),
                                               hs.data_ptr(), cs.data_ptr(), _p(gates), st), "lstm_step_fwd")
         if need_grad:
-            ctx.save_for_backward(xo, s_gate, h0c, c0c, hs, cs, gates, wx, *wpt)
+            ctx.dims = (n, b, t_len, c_in, n_layers, hid)
+            ctx.save_for_backward(xo, s_gate, h0, c0, hs, cs, gates, wx, *wpt)
         h_top = hs[n_layers - 1, t_len - 1].view(n, b, hid)
         if want_state:
             h_n, c_n = hs[:, t_len - 1], cs[:, t_len - 1]
@@ -586,15 +615,11 @@ class SharedLSTM(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, d_top, _dhn, _dcn):
-        n, b, t_len, c_in, n_layers, hid = ctx.dims
-        if ctx.planes16:
-            xo, s_gate = ctx.saved_tensors
-            d_s, w_grads = _lstm16_backward(xo, s_gate, ctx.tape16, n_layers, ctx.planes, d_top)
-            return (None, d_s, None, None, None, None, None, *w_grads)
         if getattr(ctx, "tape_consumed", False):
             raise RuntimeError("SharedLSTM (exact-fp32 kernels): the gate tape was overwritten in place by the first backward "
                                "pass; a second backward over the same graph is not supported on this path")
         ctx.tape_consumed = True
+        n, b, t_len, c_in, n_layers, hid = ctx.dims
         xo, s_gate, h0, c0, hs, cs, gates, wx, *wpt = ctx.saved_tensors
         rows = n * b
         dev = xo.device
@@ -622,6 +647,26 @@ class SharedLSTM(torch.autograd.Function):
                                            dwp[l].data_ptr(), st), "lstm_wgrad")
         w_grads = _unpack_lstm_grads(dwx, dwp, dbp, n_layers, hid, c_in)
         return (None, d_s, None, None, None, None, None, *w_grads)
+
+
+class SharedLSTM:
+    """h_top (N,B,H) of the shared multi-layer LSTM over rows r = n*B + b; input ``xo * s[b,t]``.
+
+    apply(xo (N,B,T,C), s (B,T), h0|None, c0|None (L,R,H), n_layers, hid, want_state, *lstm_weights) where
+    lstm_weights = [w_ih_l0, w_hh_l0, b_ih_l0, b_hh_l0, w_ih_l1, ...] (nn.LSTM names/shapes).
+    Returns (h_top, h_n (L,R,H), c_n (L,R,H)); the last two are not differentiable.
+
+    Picks one of two kernel families (include/stmgcn_b200.h), each its own autograd Function:
+    * H = 64, C <= 4, T <= 64 (the reference's configuration, Main.py:62) and ``lstm_path() == "tc"``:
+      :class:`SharedLSTM16`, the tcgen05 bf16-plane kernels;
+    * anything else, or ``lstm_path() == "fma"``: :class:`SharedLSTMExact`, the exact-fp32 CUDA-core kernels.
+    """
+
+    @staticmethod
+    def apply(xo, s_gate, h0, c0, n_layers: int, hid: int, want_state: bool, *weights):
+        _, _, t_len, c_in = xo.shape
+        fn = SharedLSTM16 if hid == 64 and lstm_path() == "tc" and c_in <= 4 and t_len <= 64 else SharedLSTMExact
+        return fn.apply(xo, s_gate, h0, c0, n_layers, hid, want_state, *weights)
 
 
 class FuseOut(torch.autograd.Function):

@@ -39,11 +39,25 @@ def test_library_exports_every_declared_symbol():
 
 def test_c_abi_argument_errors_come_back_as_codes_with_a_message():
     """The C entry points validate their arguments before touching CUDA: a bad call returns a negative code and
-    stmgcn_last_error() explains it (no GPU needed).  Covers the entries added in ABI 3."""
+    stmgcn_last_error() explains it (no GPU needed).  Covers the entries added in ABI 3 and 4."""
     import ctypes
     from stmgcn_b200 import _lib
     lib = _lib.lib
     null = ctypes.c_void_p(0)
+    # tensor-core projection: each entry runs its kernels or rejects the call (no quiet FFMA fallback).  The fake device
+    # pointers are never dereferenced: validation fails first.
+    ok, odd = ctypes.c_void_p(256), ctypes.c_void_p(4)
+    err_arg, err_shape, err_align = -1, -2, -3
+
+    def fwd_tc(ks=3, s=ok, out=ok):
+        return lib.stmgcn_proj_fwd_tc(s, 128 * 64, ks, 128, ok, null, _lib.ACT_RELU, out, null)
+
+    def bwd_tc(ks=3, s=ok, u=ok):
+        return lib.stmgcn_proj_bwd_tc(s, 128 * 64, ks, 128, ok, _lib.ACT_RELU, ok, ok, ok, ok, null, u, 128 * 64, null)
+
+    for name, call, null_arg in (("proj_fwd_tc", fwd_tc, "out"), ("proj_bwd_tc", bwd_tc, "u")):
+        for kwargs, code in (({"ks": 9}, err_shape), ({null_arg: null}, err_arg), ({"s": odd}, err_align)):
+            assert call(**kwargs) == code and name.encode() in lib.stmgcn_last_error(), (name, kwargs)
     # time-fused LSTM backward: null workspaces
     rc = lib.stmgcn_lstm16_layer_bwd(0, 12, 3, 128, 1, 8, 2, *([null] * 18))
     assert rc < 0 and b"lstm16_layer_bwd" in lib.stmgcn_last_error()

@@ -157,8 +157,8 @@ def test_lstm_tensor_core_vs_exact_fp32_at_cfg3_size():
         ops.set_lstm_path(old)
     names = ["h_top", "d_s"] + [f"w{i}" for i in range(4 * lyr)]
     # weight gradients are sums over 3.1 M (row, step) pairs: the two kernels add them in different orders in fp32, which
-    # alone is worth ~1e-4 relative (measured 9.4e-5 between the 3xTF32 kernels and the FFMA kernels); the fp64-oracle tests
-    # above are the pin, this one guards against indexing bugs at > 2^31-element sizes
+    # alone is worth ~1e-4 relative (measured 9.4e-5 between the first-generation 3xTF32 LSTM kernels and the FFMA
+    # kernels); the fp64-oracle tests above are the pin, this one guards against indexing bugs at > 2^31-element sizes
     for name, a, c in zip(names, res["tc"], res["fma"]):
         assert_close(a.cpu().numpy(), c.cpu().numpy(), f"cfg3-size tc vs fma {name}", 5e-5 if name in ("h_top",) else 3e-4)
 

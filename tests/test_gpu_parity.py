@@ -216,7 +216,7 @@ def test_errors_are_loud():
 
 @pytest.mark.parametrize("rows_n,b,t,c", [(5, 60, 3, 1), (3, 50, 2, 2), (40, 64, 4, 1), (7, 36, 8, 1), (2, 1100, 4, 1)])
 def test_lstm_tensor_core_path_matches_exact_fp32_path(rows_n, b, t, c):
-    """tcgen05 3xTF32 LSTM forward vs the exact-FFMA kernels on the same inputs (ragged 128-row tiles)."""
+    """tcgen05 bf16-plane (3xBF16) LSTM forward vs the exact-FFMA kernels on the same inputs (ragged 128-row tiles)."""
     from stmgcn_b200 import ops
     hid, lyr = 64, 3
     gen = torch.Generator().manual_seed(rows_n * 100 + t)
@@ -248,7 +248,7 @@ def test_lstm_tensor_core_path_matches_exact_fp32_path(rows_n, b, t, c):
 @pytest.mark.parametrize("rows_n,b,t,c", [(5, 60, 3, 1), (40, 64, 4, 1), (3, 50, 2, 2), (7, 36, 8, 1), (2, 1100, 4, 1)])
 def test_lstm_tensor_core_backward_matches_exact_fp32_path(rows_n, b, t, c):
     """tcgen05 fused BPTT kernel (pointwise in the loader + dA.Wp^T) vs the exact-FFMA kernels: d_s and all
-    LSTM weight gradients (C=2 exercises the mixed case: layer 0 on FFMA, layers > 0 on tensor cores)."""
+    LSTM weight gradients (C=2 exercises the tensor-core kernels' multi-channel layer-0 input; they cover C <= 4)."""
     from stmgcn_b200 import ops
     hid, lyr = 64, 3
     gen = torch.Generator().manual_seed(7 + rows_n)
