@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define STMGCN_ABI_VERSION 4
+#define STMGCN_ABI_VERSION 5
 
 /* error codes < 0 */
 #define STMGCN_ERR_ARG      (-1)   /* null pointer / bad enum */
@@ -134,7 +134,7 @@ int32_t stmgcn_gate_fwd(const float* pool, int64_t b, int32_t t, int64_t n_regio
 int32_t stmgcn_gate_bwd(const float* d_s, const float* z, const float* a1, const float* s, int64_t b,
                         int32_t t, const float* fcw, float* d_fcw, float* d_fcb, float* d_z, void* stream);
 
-/* ---- K3b (exact fp32, any H <= 128): shared-weight LSTM, one call per timestep (STMGCN.py:44, :47-50) ------------
+/* ---- K3b (exact fp32, any H <= 128): shared-weight LSTM, one call per direction (STMGCN.py:44, :47-50) ------------
  * The CUDA-core path for every shape the tensor-core kernels below do not cover (H != 64 or C > 4), and the on-device
  * reference the parity tests compare them with.  Weights are passed packed, H = hid, columns gate-interleaved
  * col = 4*unit + gate (gate order i,f,g,o):
@@ -146,34 +146,32 @@ int32_t stmgcn_gate_bwd(const float* d_s, const float* z, const float* a1, const
  *   hs, cs: (L, T, R, H);  gates: (L, T, R, 4H) post-activation, gate-interleaved (NULL in inference);
  * xo: (R, T, C) node-major observations, s_gate: (B, T) context gate (the modulation xo * s is fused into the layer-0
  * input read, STMGCN.py:44).  h0/c0: (L, R, H) or NULL (zeros, STMGCN.py:53-57).
- * Step t computes layers 0..L-1.  Limits: H % 4 == 0, H <= 128, C <= 4, L <= 8. */
-int32_t stmgcn_lstm_step_fwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                             int32_t c_in, int64_t b_inner, const float* xo, const float* s_gate,
-                             const float* wx, const float* const* wp, const float* const* bp,
-                             const float* h0, const float* c0, float* hs, float* cs, float* gates, void* stream);
-/* BPTT step t (call t = T-1 .. 0).  d_top: (R, H) gradient of hs[L-1][T-1] (read at t = T-1 only).
- * Workspaces: dh_rec, dc: (L, R, H); dx_work: (R, H).  No initialisation is needed: the call with t = T-1 treats the
- * incoming dh_rec / dc as zero without reading them (h_n / c_n carry no gradient, STMGCN.py:113).
- * gates[l][t] is overwritten IN PLACE with the pre-activation gradients dA (stmgcn_lstm_wgrad reads them).
- * Accumulates (+=; caller zeroes): d_s (B,T) = sum_{n,c} dxmod * xo (gate adjoint, STMGCN.py:44),
- * dwx (C,4H), dbp[l] (4H). */
-int32_t stmgcn_lstm_step_bwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                             int32_t c_in, int64_t b_inner, const float* xo, const float* s_gate,
-                             const float* wx, const float* const* wpt, const float* c0, const float* cs,
-                             float* gates, const float* d_top, float* dh_rec, float* dc, float* dx_work,
-                             float* d_s, float* dwx, float* const* dbp, void* stream);
-/* weight gradients of one layer after all stmgcn_lstm_step_bwd calls:
- * dwp (kd_l, 4H) += [h_below_t | h_{t-1}]^T dA summed over all (t, r). */
-int32_t stmgcn_lstm_wgrad(int32_t layer, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                          const float* h0, const float* hs, const float* gates_da, float* dwp, void* stream);
+ * The forward runs every timestep t = 0 .. T-1, layers 0..L-1 within a step.  Limits: H % 4 == 0, H <= 128, C <= 4,
+ * L <= 8. */
+int32_t stmgcn_lstm_fwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid, int32_t c_in, int64_t b_inner,
+                        const float* xo, const float* s_gate, const float* wx, const float* const* wp,
+                        const float* const* bp, const float* h0, const float* c0, float* hs, float* cs, float* gates,
+                        void* stream);
+/* BPTT through all timesteps t = T-1 .. 0 (layers top-down within a step), then the weight gradients layer by layer.
+ * d_top: (R, H) gradient of hs[L-1][T-1].  Workspaces (none needs initialisation; h_n / c_n carry no gradient,
+ * STMGCN.py:113): dh_rec, dc: (L, R, H); dx_work: (R, H).
+ * gates is overwritten IN PLACE with the pre-activation gradients dA: the tape serves one backward only.
+ * Accumulates (+=; caller zeroes): d_s (B,T) = sum_{n,c} dxmod * xo (gate adjoint, STMGCN.py:44), dwx (C,4H),
+ * dbp[l] (4H), dwp[l] (kd_l, 4H) = [h_below_t | h_{t-1}]^T dA summed over all (t, r). */
+int32_t stmgcn_lstm_bwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid, int32_t c_in, int64_t b_inner,
+                        const float* xo, const float* s_gate, const float* wx, const float* const* wpt, const float* h0,
+                        const float* c0, const float* hs, const float* cs, float* gates, const float* d_top,
+                        float* dh_rec, float* dc, float* dx_work, float* d_s, float* dwx, float* const* dbp,
+                        float* const* dwp, void* stream);
 
 /* ---- K3b on the tensor cores (H = 64, C <= 4): bf16-plane LSTM without a gate tape -----------------------------
- * Same arithmetic contract as stmgcn_lstm_step_fwd/_bwd/_wgrad (STMGCN.py:44, :47-50; nn.LSTM semantics, fp32 state and
+ * Same arithmetic contract as stmgcn_lstm_fwd / _bwd (STMGCN.py:44, :47-50; nn.LSTM semantics, fp32 state and
  * accumulation), different tape:
  *   hp : (L, T, P, R, 64) bf16 -- every hidden state as P planes; P = 2: hi = bf16(h), lo = bf16(h - hi) (3-pass
  *        "3xBF16" products, ~2^-18 operand error: fp32-grade, the 1e-4 parity bar holds with >10x margin);
  *        P = 1: hi only, single-pass bf16 products (the arithmetic of the bf16-quoted BASELINE configs).
- *   cs : (L, T, ceil(R/128)*128, 64) fp32, tile-blocked (element (r,u) at (((r/128)*16 + u/4)*128 + r%128)*4 + u%4).
+ *   cs : (L, T, R_pad, 64) fp32, R_pad = ceil(R/128)*128, tile-blocked (element (r,u) at
+ *        (((r/128)*16 + u/4)*128 + r%128)*4 + u%4).
  * No gate tape: the backward recomputes the gates from hp (which it needs anyway for the weight gradients).
  * stmgcn_lstm16_pack turns one layer's nn.LSTM parameters (native layout: w_ih (256, in), w_hh (256, 64), b_ih, b_hh
  * (256), gate order i,f,g,o) into the resident operand image wimg (layer 0: 64 KB, layers > 0: 128 KB; tiles
@@ -181,40 +179,39 @@ int32_t stmgcn_lstm_wgrad(int32_t layer, int32_t t_len, int32_t n_layers, int64_
  * gate-interleaved (col = 4*unit + gate) and, for layer 0, wih_t (C, 256) = W_ih^T gate-interleaved. */
 int32_t stmgcn_lstm16_pack(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, int32_t layer,
                            int32_t c_in, void* wimg, float* bias, float* wih_t, void* stream);
-/* One timestep, all layers.  h0p: (L, P, R, 64) bf16 planes of the initial hidden state and c0: (L, R_pad, 64) fp32
- * tile-blocked, or both NULL (zeros, STMGCN.py:53-57).  At t = T-1 the fp32 hidden state is also written: every layer
- * into h_n (L, R, 64) when h_n != NULL, else only the top layer into h_top (R, 64) -- the (N,B,H) operand of the
- * spatial GCN (STMGCN.py:50, :114).  C <= 4. */
-int32_t stmgcn_lstm16_step_fwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in,
-                               int64_t b_inner, int32_t planes, const float* xo, const float* s_gate,
-                               const void* const* wimg, const float* const* bias, const float* wih_t,
-                               const void* h0p, const float* c0, void* hp, float* cs, float* h_top, float* h_n,
-                               void* stream);
+/* The forward through all timesteps t = 0 .. T-1, layers 0..L-1 within a step (one launch per layer-step).
+ * wimg[l] / bias[l]: layer l's operands from stmgcn_lstm16_pack.  h0p: (L, P, R, 64) bf16 planes of the initial hidden
+ * state and c0: (L, R_pad, 64) fp32 tile-blocked, or both NULL (zeros, STMGCN.py:53-57).  At t = T-1 the fp32 hidden
+ * state is also written: every layer into h_n (L, R, 64) when h_n != NULL, else only the top layer into h_top (R, 64) --
+ * the (N,B,H) operand of the spatial GCN (STMGCN.py:50, :114).  C <= 4, L <= 8. */
+int32_t stmgcn_lstm16_fwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in, int64_t b_inner, int32_t planes,
+                          const float* xo, const float* s_gate, const void* const* wimg, const float* const* bias,
+                          const float* wih_t, const void* h0p, const float* c0, void* hp, float* cs, float* h_top,
+                          float* h_n, void* stream);
 
 /* grid (CTAs) the lstm16 kernels use for `rows` rows: the number of weight-gradient scratch slices per layer */
 int32_t stmgcn_lstm16_grid(int64_t rows);
-/* BPTT of ONE layer through all timesteps T-1 .. 0 (call the layers top-down): recomputes the gates from hp, forms dA,
- * accumulates the weight and bias gradients and propagates [dx_below | dh_prev].  A tile's rows never mix with other
- * tiles', so each CTA walks its own tiles through time inside a launch; a launch covers as many consecutive timesteps as
- * keep a CTA's weight-gradient accumulation chain within 6144 rows (cfg3: 3 steps, 4 launches per layer).  T <= 64.
- * Workspaces (tile-blocked, R_pad = ceil(R/128)*128 rows; none needs initialisation):
- *   dh_in : top layer: d_top (R_pad,64), the gradient of the top layer's last hidden state; other layers: the dx_out
- *           (T,R_pad,64) the layer above wrote;      dx_out: (T,R_pad,64), NULL for layer 0;
- *   dh_rec, dc: (R_pad,64) scratch of this layer;    dw_scratch: (stmgcn_lstm16_grid(rows), 128*256) floats;
- *   zero_tile: 16 KB of zeros (the h_prev operand at t = 0 without an initial state).
- * wimg / bias: this layer's operands from stmgcn_lstm16_pack.  Accumulates (+=; caller zeroes): d_s (B,T), dbp (256,
- * gate-interleaved). */
-int32_t stmgcn_lstm16_layer_bwd(int32_t layer, int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in,
-                                int64_t b_inner, int32_t planes, const float* xo, const float* s_gate,
-                                const void* wimg, const float* bias, const float* wih_t, const void* h0p,
-                                const float* c0, const void* hp, const float* cs, const float* dh_in,
-                                float* dx_out, float* dh_rec, float* dc, float* d_s, float* dbp,
-                                float* dw_scratch, const void* zero_tile, void* stream);
-/* After stmgcn_lstm16_layer_bwd of layer `layer`: sum its scratch slices into nn.LSTM-native gradients
- * d_w_ih (256, in), d_w_hh (256, 64), d_b_ih = d_b_hh (256) (overwritten, not accumulated). */
-int32_t stmgcn_lstm16_wgrad_reduce(int32_t layer, int32_t c_in, int32_t n_slices, const float* slices,
-                                   const float* dbp, float* d_w_ih, float* d_w_hh, float* d_b_ih, float* d_b_hh,
-                                   void* stream);
+/* BPTT through all timesteps, layers top-down, then one reduction per layer into the nn.LSTM-native gradients.  Per
+ * layer the kernel recomputes the gates from hp, forms dA, accumulates the weight and bias gradients and propagates
+ * [dx_below | dh_prev].  A tile's rows never mix with other tiles', so each CTA walks its own tiles through time inside
+ * a launch; a launch covers as many consecutive timesteps as keep a CTA's weight-gradient accumulation chain within
+ * 6144 rows (cfg3: 3 steps, 4 launches per layer).  T <= 64, C <= 4, L <= 8.
+ * Inputs: those of stmgcn_lstm16_fwd and its tape hp, cs; d_top (R_pad, 64) tile-blocked, the gradient of the top
+ * layer's last hidden state.
+ * Workspaces (fp32, tile-blocked where they have R_pad rows):
+ *   dh_rec, dc : (R_pad, 64), no initialisation needed;
+ *   dx_work    : min(2, L-1) slices of (T, R_pad, 64), no initialisation needed; NULL exactly when L == 1 (the gradient
+ *                a layer passes to the layer below, for every step);
+ *   dbp        : (L, 256) and d_s (B, T), both ZEROED by the caller; d_s receives the gate adjoint (STMGCN.py:44);
+ *   dw_scratch : (L, stmgcn_lstm16_grid(rows), 128*256), no initialisation needed;
+ *   zero_tile  : 16 KB of zeros (the h_prev operand at t = 0 without an initial state).
+ * grads: 4*L device pointers in nn.LSTM parameter order, per layer d_w_ih (256, in_l), d_w_hh (256, 64), d_b_ih (256),
+ * d_b_hh (256) (in_0 = C, else 64); overwritten, not accumulated. */
+int32_t stmgcn_lstm16_bwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in, int64_t b_inner, int32_t planes,
+                          const float* xo, const float* s_gate, const void* const* wimg, const float* const* bias,
+                          const float* wih_t, const void* h0p, const float* c0, const void* hp, const float* cs,
+                          const float* d_top, float* dh_rec, float* dc, float* dx_work, float* d_s, float* dbp,
+                          float* dw_scratch, const void* zero_tile, float* const* grads, void* stream);
 
 /* ---- fusion over graphs + output FC (STMGCN.py:116-118) ------------------------------------------
  * feat = sum_m g[m] (each (R, G) node-major); y[b, n, c] = feat[n*B+b, :] . fcw[c, :] + fcb[c]. */

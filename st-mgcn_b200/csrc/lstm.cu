@@ -232,9 +232,9 @@ lstm_bwd_pointwise_kernel(int64_t rows, int hid, float* __restrict__ gates, cons
     }
 }
 
-int32_t check_dims(const char* who, int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                   int32_t c_in, int64_t b_inner) {
-    STMGCN_REQUIRE(t >= 0 && t < t_len, STMGCN_ERR_SHAPE, "%s: t=%d out of [0,%d)", who, t, t_len);
+int32_t check_dims(const char* who, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid, int32_t c_in,
+                   int64_t b_inner) {
+    STMGCN_REQUIRE(t_len >= 1, STMGCN_ERR_SHAPE, "%s: T=%d", who, t_len);
     STMGCN_REQUIRE(n_layers >= 1 && n_layers <= kMaxLayers, STMGCN_ERR_SHAPE, "%s: layers=%d (max %d)", who,
                    n_layers, kMaxLayers);
     STMGCN_REQUIRE(rows > 0 && b_inner > 0 && rows % b_inner == 0, STMGCN_ERR_SHAPE, "%s: rows=%lld b=%lld", who,
@@ -250,144 +250,142 @@ int32_t check_dims(const char* who, int32_t t, int32_t t_len, int32_t n_layers, 
 
 extern "C" {
 
-int32_t stmgcn_lstm_step_fwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                             int32_t c_in, int64_t b_inner, const float* xo, const float* s_gate,
-                             const float* wx, const float* const* wp, const float* const* bp,
-                             const float* h0, const float* c0, float* hs, float* cs, float* gates, void* stream) {
-    STMGCN_REQUIRE(xo && s_gate && wx && wp && bp && hs && cs, STMGCN_ERR_ARG, "lstm_step_fwd: null pointer");
-    if (int32_t rc = check_dims("lstm_step_fwd", t, t_len, n_layers, rows, hid, c_in, b_inner)) return rc;
+int32_t stmgcn_lstm_fwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid, int32_t c_in, int64_t b_inner,
+                        const float* xo, const float* s_gate, const float* wx, const float* const* wp,
+                        const float* const* bp, const float* h0, const float* c0, float* hs, float* cs, float* gates,
+                        void* stream) {
+    STMGCN_REQUIRE(xo && s_gate && wx && wp && bp && hs && cs, STMGCN_ERR_ARG, "lstm_fwd: null pointer");
+    if (int32_t rc = check_dims("lstm_fwd", t_len, n_layers, rows, hid, c_in, b_inner)) return rc;
+    for (int l = 0; l < n_layers; ++l) STMGCN_REQUIRE(wp[l] && bp[l], STMGCN_ERR_ARG, "lstm_fwd: wp/bp[%d] null", l);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t rh = rows * hid;
     const int h4 = 4 * hid;
-    for (int l = 0; l < n_layers; ++l) {
-        STMGCN_REQUIRE(wp[l] && bp[l], STMGCN_ERR_ARG, "lstm_step_fwd: wp/bp[%d] null", l);
-        const float* h_prev = t > 0 ? hs + ((int64_t)(l * t_len + t - 1)) * rh : (h0 ? h0 + (int64_t)l * rh : nullptr);
-        const float* c_prev = t > 0 ? cs + ((int64_t)(l * t_len + t - 1)) * rh : (c0 ? c0 + (int64_t)l * rh : nullptr);
-        ASegs a{};
-        a.segw = hid;
-        a.lda = hid;
-        if (l == 0) {
-            a.nseg = 1;
-            a.seg[0] = h_prev;
-        } else {
-            a.nseg = 2;
-            a.seg[0] = hs + ((int64_t)((l - 1) * t_len + t)) * rh;
-            a.seg[1] = h_prev;
+    for (int t = 0; t < t_len; ++t)
+        for (int l = 0; l < n_layers; ++l) {
+            const float* h_prev = t > 0 ? hs + ((int64_t)(l * t_len + t - 1)) * rh : (h0 ? h0 + (int64_t)l * rh : nullptr);
+            const float* c_prev = t > 0 ? cs + ((int64_t)(l * t_len + t - 1)) * rh : (c0 ? c0 + (int64_t)l * rh : nullptr);
+            ASegs a{};
+            a.segw = hid;
+            a.lda = hid;
+            if (l == 0) {
+                a.nseg = 1;
+                a.seg[0] = h_prev;
+            } else {
+                a.nseg = 2;
+                a.seg[0] = hs + ((int64_t)((l - 1) * t_len + t)) * rh;
+                a.seg[1] = h_prev;
+            }
+            LstmCellEpi epi;
+            epi.bias = bp[l];
+            epi.wx = (l == 0) ? wx : nullptr;
+            epi.xo = xo;
+            epi.sg = s_gate;
+            epi.c_in = c_in;
+            epi.t = t;
+            epi.t_len = t_len;
+            epi.b_inner = b_inner;
+            epi.c_prev = c_prev;
+            epi.h_out = hs + ((int64_t)(l * t_len + t)) * rh;
+            epi.c_out = cs + ((int64_t)(l * t_len + t)) * rh;
+            epi.gates_out = gates ? gates + ((int64_t)(l * t_len + t)) * rows * h4 : nullptr;
+            epi.hid = hid;
+            epi.half_units = 256 / 8;
+            const int kd = a.nseg * hid;
+            int32_t rc;
+            if (vec_ok(a, wp[l], h4, h4))
+                rc = launch_tall<256, true>(a, rows, kd, wp[l], h4, h4, epi, st, "lstm_fwd");
+            else
+                rc = launch_tall<256, false>(a, rows, kd, wp[l], h4, h4, epi, st, "lstm_fwd");
+            if (rc) return rc;
         }
-        LstmCellEpi epi;
-        epi.bias = bp[l];
-        epi.wx = (l == 0) ? wx : nullptr;
-        epi.xo = xo;
-        epi.sg = s_gate;
-        epi.c_in = c_in;
-        epi.t = t;
-        epi.t_len = t_len;
-        epi.b_inner = b_inner;
-        epi.c_prev = c_prev;
-        epi.h_out = hs + ((int64_t)(l * t_len + t)) * rh;
-        epi.c_out = cs + ((int64_t)(l * t_len + t)) * rh;
-        epi.gates_out = gates ? gates + ((int64_t)(l * t_len + t)) * rows * h4 : nullptr;
-        epi.hid = hid;
-        epi.half_units = 256 / 8;
-        const int kd = a.nseg * hid;
-        int32_t rc;
-        if (vec_ok(a, wp[l], h4, h4))
-            rc = launch_tall<256, true>(a, rows, kd, wp[l], h4, h4, epi, st, "lstm_step_fwd");
-        else
-            rc = launch_tall<256, false>(a, rows, kd, wp[l], h4, h4, epi, st, "lstm_step_fwd");
-        if (rc) return rc;
-    }
     return 0;
 }
 
-int32_t stmgcn_lstm_step_bwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                             int32_t c_in, int64_t b_inner, const float* xo, const float* s_gate,
-                             const float* wx, const float* const* wpt, const float* c0, const float* cs, float* gates,
-                             const float* d_top, float* dh_rec, float* dc, float* dx_work, float* d_s, float* dwx,
-                             float* const* dbp, void* stream) {
-    STMGCN_REQUIRE(xo && s_gate && wx && wpt && cs && gates && dh_rec && dc && dx_work && d_s && dwx && dbp,
-                   STMGCN_ERR_ARG, "lstm_step_bwd: null pointer");
-    if (int32_t rc = check_dims("lstm_step_bwd", t, t_len, n_layers, rows, hid, c_in, b_inner)) return rc;
+int32_t stmgcn_lstm_bwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid, int32_t c_in, int64_t b_inner,
+                        const float* xo, const float* s_gate, const float* wx, const float* const* wpt, const float* h0,
+                        const float* c0, const float* hs, const float* cs, float* gates, const float* d_top,
+                        float* dh_rec, float* dc, float* dx_work, float* d_s, float* dwx, float* const* dbp,
+                        float* const* dwp, void* stream) {
+    STMGCN_REQUIRE(xo && s_gate && wx && wpt && hs && cs && gates && d_top && dh_rec && dc && dx_work && d_s && dwx && dbp &&
+                       dwp,
+                   STMGCN_ERR_ARG, "lstm_bwd: null pointer");
+    if (int32_t rc = check_dims("lstm_bwd", t_len, n_layers, rows, hid, c_in, b_inner)) return rc;
+    for (int l = 0; l < n_layers; ++l)
+        STMGCN_REQUIRE(wpt[l] && dbp[l] && dwp[l], STMGCN_ERR_ARG, "lstm_bwd: wpt/dbp/dwp[%d] null", l);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t rh = rows * hid;
     const int h4 = 4 * hid;
     const int grid_pw = (int)((ceil_div(rows, 8) < (int64_t)sm_count() * 4) ? ceil_div(rows, 8) : (int64_t)sm_count() * 4);
-    for (int l = n_layers - 1; l >= 0; --l) {
-        STMGCN_REQUIRE(wpt[l] && dbp[l], STMGCN_ERR_ARG, "lstm_step_bwd: wpt/dbp[%d] null", l);
-        float* g_lt = gates + ((int64_t)(l * t_len + t)) * rows * h4;
-        const float* c_t = cs + ((int64_t)(l * t_len + t)) * rh;
-        const float* c_prev = t > 0 ? cs + ((int64_t)(l * t_len + t - 1)) * rh : (c0 ? c0 + (int64_t)l * rh : nullptr);
-        const float* dh_in = (l == n_layers - 1) ? ((t == t_len - 1) ? d_top : nullptr) : dx_work;
-        const bool l0 = (l == 0);
-        size_t smem = (size_t)h4 * (1 + (l0 ? c_in : 0)) * sizeof(float);
-        if (l0 && b_inner <= 2048) smem += (size_t)b_inner * sizeof(float);
-        lstm_bwd_pointwise_kernel<<<grid_pw, 256, smem, st>>>(
-            rows, hid, g_lt, c_t, c_prev, dh_in, dh_rec + (int64_t)l * rh, dc + (int64_t)l * rh, dbp[l],
-            l0 ? wx : nullptr, l0 ? dwx : nullptr, xo, s_gate, d_s, c_in, t, t_len, b_inner);
-        count_launch();
-        if (int32_t rc = check_launch("lstm_bwd_pointwise")) return rc;
-        // data gradients: [dx_below | dh_rec] = dA . wpt[l]      (dA: rows x 4H, wpt[l]: 4H x kd_l)
-        ASegs a{};
-        a.nseg = 1;
-        a.segw = h4;
-        a.lda = h4;
-        a.seg[0] = g_lt;
-        StoreSplitEpi epi;
-        epi.dst0 = l0 ? nullptr : dx_work;
-        epi.ld0 = hid;
-        epi.w0 = l0 ? 0 : hid;
-        epi.dst1 = dh_rec + (int64_t)l * rh;
-        epi.ld1 = hid;
-        const int nc = l0 ? hid : 2 * hid;
-        int32_t rc;
-        if (nc > 64) {
-            epi.half_cols = 64;
-            if (vec_ok(a, wpt[l], nc, nc)) rc = launch_tall<128, true>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd_data");
-            else rc = launch_tall<128, false>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd_data");
-        } else {
-            epi.half_cols = 32;
-            if (vec_ok(a, wpt[l], nc, nc)) rc = launch_tall<64, true>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd_data");
-            else rc = launch_tall<64, false>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd_data");
+    // BPTT, t = T-1 .. 0, layers top-down; dx_work carries a layer's input gradient to the layer below
+    for (int t = t_len - 1; t >= 0; --t)
+        for (int l = n_layers - 1; l >= 0; --l) {
+            float* g_lt = gates + ((int64_t)(l * t_len + t)) * rows * h4;
+            const float* c_t = cs + ((int64_t)(l * t_len + t)) * rh;
+            const float* c_prev = t > 0 ? cs + ((int64_t)(l * t_len + t - 1)) * rh : (c0 ? c0 + (int64_t)l * rh : nullptr);
+            const float* dh_in = (l == n_layers - 1) ? ((t == t_len - 1) ? d_top : nullptr) : dx_work;
+            const bool l0 = (l == 0);
+            size_t smem = (size_t)h4 * (1 + (l0 ? c_in : 0)) * sizeof(float);
+            if (l0 && b_inner <= 2048) smem += (size_t)b_inner * sizeof(float);
+            lstm_bwd_pointwise_kernel<<<grid_pw, 256, smem, st>>>(
+                rows, hid, g_lt, c_t, c_prev, dh_in, dh_rec + (int64_t)l * rh, dc + (int64_t)l * rh, dbp[l],
+                l0 ? wx : nullptr, l0 ? dwx : nullptr, xo, s_gate, d_s, c_in, t, t_len, b_inner);
+            count_launch();
+            if (int32_t rc = check_launch("lstm_bwd (pointwise)")) return rc;
+            // data gradients: [dx_below | dh_rec] = dA . wpt[l]      (dA: rows x 4H, wpt[l]: 4H x kd_l)
+            ASegs a{};
+            a.nseg = 1;
+            a.segw = h4;
+            a.lda = h4;
+            a.seg[0] = g_lt;
+            StoreSplitEpi epi;
+            epi.dst0 = l0 ? nullptr : dx_work;
+            epi.ld0 = hid;
+            epi.w0 = l0 ? 0 : hid;
+            epi.dst1 = dh_rec + (int64_t)l * rh;
+            epi.ld1 = hid;
+            const int nc = l0 ? hid : 2 * hid;
+            int32_t rc;
+            if (nc > 64) {
+                epi.half_cols = 64;
+                if (vec_ok(a, wpt[l], nc, nc)) rc = launch_tall<128, true>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd (data)");
+                else rc = launch_tall<128, false>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd (data)");
+            } else {
+                epi.half_cols = 32;
+                if (vec_ok(a, wpt[l], nc, nc)) rc = launch_tall<64, true>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd (data)");
+                else rc = launch_tall<64, false>(a, rows, h4, wpt[l], nc, nc, epi, st, "lstm_bwd (data)");
+            }
+            if (rc) return rc;
         }
+    // weight gradients, one layer at a time: dwp[l] += [h_below_t | h_{t-1}]^T dA summed over all (t, r)
+    for (int l = 0; l < n_layers; ++l) {
+        ASegs a{};
+        ReduceTime tm{};
+        a.segw = hid;
+        a.lda = hid;
+        tm.n_t = t_len;
+        tm.d_tstride = rows * h4;
+        int s = 0;
+        if (l > 0) {                           // input from the layer below, same step
+            a.seg[s] = hs + ((int64_t)(l - 1) * t_len) * rh;
+            tm.a_tstride[s] = rh;
+            tm.a_shift[s] = 0;
+            tm.a_t0[s] = nullptr;
+            ++s;
+        }
+        a.seg[s] = hs + ((int64_t)l * t_len) * rh;      // h_{t-1} of this layer
+        tm.a_tstride[s] = rh;
+        tm.a_shift[s] = 1;
+        tm.a_t0[s] = h0 ? h0 + (int64_t)l * rh : nullptr;
+        ++s;
+        a.nseg = s;
+        const int kd = s * hid;
+        const float* d = gates + ((int64_t)l * t_len) * rows * h4;
+        const bool vec = (hid % 4 == 0) && aligned16(d) && aligned16(hs) && (!h0 || aligned16(h0));
+        const int32_t rc = vec ? launch_reduce<256, true>(a, tm, rows, kd, d, h4, h4, dwp[l], h4, st, "lstm_bwd (weights)")
+                               : launch_reduce<256, false>(a, tm, rows, kd, d, h4, h4, dwp[l], h4, st, "lstm_bwd (weights)");
         if (rc) return rc;
     }
     return 0;
-}
-
-int32_t stmgcn_lstm_wgrad(int32_t layer, int32_t t_len, int32_t n_layers, int64_t rows, int32_t hid,
-                          const float* h0, const float* hs, const float* gates_da, float* dwp, void* stream) {
-    STMGCN_REQUIRE(hs && gates_da && dwp, STMGCN_ERR_ARG, "lstm_wgrad: null pointer");
-    STMGCN_REQUIRE(layer >= 0 && layer < n_layers && n_layers <= kMaxLayers && t_len > 0 && rows > 0 && hid > 0 &&
-                       hid % 4 == 0,
-                   STMGCN_ERR_SHAPE, "lstm_wgrad: bad shape");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t rh = rows * hid;
-    const int h4 = 4 * hid;
-    ASegs a{};
-    ReduceTime tm{};
-    a.segw = hid;
-    a.lda = hid;
-    tm.n_t = t_len;
-    tm.d_tstride = rows * h4;
-    int s = 0;
-    if (layer > 0) {                       // input from the layer below, same step
-        a.seg[s] = hs + ((int64_t)(layer - 1) * t_len) * rh;
-        tm.a_tstride[s] = rh;
-        tm.a_shift[s] = 0;
-        tm.a_t0[s] = nullptr;
-        ++s;
-    }
-    a.seg[s] = hs + ((int64_t)layer * t_len) * rh;      // h_{t-1} of this layer
-    tm.a_tstride[s] = rh;
-    tm.a_shift[s] = 1;
-    tm.a_t0[s] = h0 ? h0 + (int64_t)layer * rh : nullptr;
-    ++s;
-    a.nseg = s;
-    const int kd = s * hid;
-    const float* d = gates_da + ((int64_t)layer * t_len) * rows * h4;
-    bool vec = (hid % 4 == 0) && aligned16(d) && aligned16(hs) && (!h0 || aligned16(h0));
-    if (vec) return launch_reduce<256, true>(a, tm, rows, kd, d, h4, h4, dwp, h4, st, "lstm_wgrad");
-    return launch_reduce<256, false>(a, tm, rows, kd, d, h4, h4, dwp, h4, st, "lstm_wgrad");
 }
 
 }  // extern "C"

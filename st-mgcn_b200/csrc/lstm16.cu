@@ -29,10 +29,6 @@
 using namespace stmgcn;
 using namespace stmgcn::tc;
 
-namespace stmgcn {
-bool make_plane_map(CUtensorMap* map, const void* base, int64_t rows, int64_t slices);
-}
-
 namespace {
 
 constexpr int kTileM = 128;
@@ -434,8 +430,8 @@ __global__ void lstm16_pack_kernel(const float* __restrict__ w_ih, const float* 
 // (4 x 32 KB) in, dc, dh_rec, dx_below (3 x 32 KB) out = 288 KB (the first-generation pair of kernels moved 640 KB).
 // Weight chunks stream from L2 twice, into one single-buffered slot for R_c and one for D_c (see the producer).
 // Partial weight gradients: every CTA adds its TMEM accumulator into its OWN slice of a scratch buffer (vector reductions,
-// no contention; the slice layout is the accumulator's register layout); stmgcn_lstm16_wgrad_reduce sums the slices once
-// per layer and writes nn.LSTM-native gradients.
+// no contention; the slice layout is the accumulator's register layout); after the last layer, stmgcn_lstm16_bwd sums the
+// slices once per layer (lstm16_wgrad_reduce_kernel) and writes nn.LSTM-native gradients.
 // The kernel is bound by the L1 / shared-memory data pipe (ncu: 94 %: tensor-core operand reads 61 % + LSU 33 %).
 constexpr int kBCompWarps = 16;
 constexpr int kBThreads = (kBCompWarps + 2) * 32;       // + MMA-issuing warp + producer warp
@@ -1129,14 +1125,10 @@ __global__ void lstm16_wgrad_reduce_kernel(const float* __restrict__ slices, int
     }
 }
 
-}  // namespace
-
-namespace stmgcn {
-
 typedef CUresult (*EncodeTiledFn16)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                     const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn16 encode_fn16() {
+EncodeTiledFn16 encode_fn16() {
     static EncodeTiledFn16 fn = nullptr;
     static bool tried = false;
     if (!tried) {
@@ -1162,21 +1154,81 @@ bool make_plane_map(CUtensorMap* map, const void* base, int64_t rows, int64_t sl
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static int32_t set_smem_attr(const void* fn, size_t bytes) { return ensure_dyn_smem(fn, bytes); }
-
 // kernel variant for (planes, cin): cin = 0 (not layer 0), 1 (layer 0, one input channel), kMaxC (layer 0, runtime count)
 using FwdFn = void (*)(const Fwd16Params);
 using BwdFn = void (*)(const Bwd16Params);
-static FwdFn fwd_kernel_for(int planes, int cin) {
+FwdFn fwd_kernel_for(int planes, int cin) {
     if (planes == 2) return cin == 0 ? lstm16_fwd_kernel<2, 0> : (cin == 1 ? lstm16_fwd_kernel<2, 1> : lstm16_fwd_kernel<2, kMaxC>);
     return cin == 0 ? lstm16_fwd_kernel<1, 0> : (cin == 1 ? lstm16_fwd_kernel<1, 1> : lstm16_fwd_kernel<1, kMaxC>);
 }
-static BwdFn bwd_kernel_for(int planes, int cin) {
+BwdFn bwd_kernel_for(int planes, int cin) {
     if (planes == 2) return cin == 0 ? lstm16_bwd_kernel<2, 0> : (cin == 1 ? lstm16_bwd_kernel<2, 1> : lstm16_bwd_kernel<2, kMaxC>);
     return cin == 0 ? lstm16_bwd_kernel<1, 0> : (cin == 1 ? lstm16_bwd_kernel<1, 1> : lstm16_bwd_kernel<1, kMaxC>);
 }
 
-}  // namespace stmgcn
+// CTAs of every lstm16 launch for `rows` rows (persistent: at most one per SM)
+int grid_for(int64_t rows) {
+    const int64_t n_tiles = ceil_div(rows, kTileM);
+    return (int)(n_tiles < sm_count() ? n_tiles : sm_count());
+}
+
+// What the forward and the backward entry check alike, before any CUDA call
+int32_t check_args(const char* who, int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in, int64_t b_inner,
+                   int32_t planes, const void* const* wimg, const float* const* bias, const void* h0p, const float* c0) {
+    STMGCN_REQUIRE(planes == 1 || planes == 2, STMGCN_ERR_ARG, "%s: planes=%d", who, planes);
+    STMGCN_REQUIRE(t_len >= 1 && n_layers >= 1 && n_layers <= 8 && rows > 0 && c_in >= 1 && c_in <= kMaxC && b_inner > 0,
+                   STMGCN_ERR_SHAPE, "%s: T=%d L=%d rows=%lld C=%d", who, t_len, n_layers, (long long)rows, c_in);
+    STMGCN_REQUIRE(rows <= (1LL << 25), STMGCN_ERR_SHAPE, "%s: rows=%lld too large (32-bit element offsets)", who, (long long)rows);
+    STMGCN_REQUIRE((h0p == nullptr) == (c0 == nullptr), STMGCN_ERR_ARG, "%s: h0p and c0 go together", who);
+    for (int l = 0; l < n_layers; ++l) STMGCN_REQUIRE(wimg[l] && bias[l], STMGCN_ERR_ARG, "%s: wimg/bias[%d] null", who, l);
+    return 0;
+}
+
+// tensor maps of the hidden-state tape hp and, when there is one, of the initial state h0p (else left zero)
+int32_t make_state_maps(const char* who, CUtensorMap* hp_map, CUtensorMap* h0_map, const void* hp, const void* h0p,
+                        int64_t rows, int t_len, int n_layers, int planes) {
+    STMGCN_REQUIRE(make_plane_map(hp_map, hp, rows, (int64_t)n_layers * t_len * planes), STMGCN_ERR_STATE,
+                   "%s: cuTensorMapEncodeTiled failed (hp)", who);
+    if (h0p != nullptr)
+        STMGCN_REQUIRE(make_plane_map(h0_map, h0p, rows, (int64_t)n_layers * planes), STMGCN_ERR_STATE,
+                       "%s: cuTensorMapEncodeTiled failed (h0p)", who);
+    return 0;
+}
+
+// The K segments of layer-step (l, t), in weight-image order ([seg0 hi | seg0 lo | seg1 hi | seg1 lo]): layers > 0 first
+// read h of the layer below at step t; every layer then reads its own h_prev -- h at t - 1, at t = 0 the initial state, or,
+// without one, zeros (STMGCN.py:53-57).  The forward leaves a zero segment out (layers > 0 then use only W_ih, layer 0 has
+// no MMA at all); the backward reads the zero tile there.
+enum : int8_t { kSegHp = 0, kSegH0 = 1, kSegZero = 2 };         // Bwd16Step::src
+struct StepPlan {
+    int nseg;
+    int8_t src[2];
+    int32_t slice[2];          // plane slice of the segment's hi plane in its tensor map (lo = + 1)
+    const float* c_prev;       // tile-blocked c_{t-1} of this layer, or nullptr (zeros)
+};
+StepPlan plan_step(int l, int t, int t_len, int planes, const float* c0, const float* cs, int64_t cslice) {
+    StepPlan s;
+    memset(&s, 0, sizeof(s));
+    if (l > 0) {
+        s.src[s.nseg] = kSegHp;
+        s.slice[s.nseg] = ((l - 1) * t_len + t) * planes;
+        ++s.nseg;
+    }
+    if (t > 0) {
+        s.src[s.nseg] = kSegHp;
+        s.slice[s.nseg] = (l * t_len + t - 1) * planes;
+    } else if (c0 != nullptr) {                                    // c0 and h0p go together
+        s.src[s.nseg] = kSegH0;
+        s.slice[s.nseg] = l * planes;
+    } else {
+        s.src[s.nseg] = kSegZero;
+    }
+    ++s.nseg;
+    s.c_prev = t > 0 ? cs + (int64_t)(l * t_len + t - 1) * cslice : (c0 ? c0 + (int64_t)l * cslice : nullptr);
+    return s;
+}
+
+}  // namespace
 
 extern "C" int32_t stmgcn_lstm16_pack(const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh,
                                       int32_t layer, int32_t c_in, void* wimg, float* bias, float* wih_t, void* stream) {
@@ -1188,135 +1240,86 @@ extern "C" int32_t stmgcn_lstm16_pack(const float* w_ih, const float* w_hh, cons
     return check_launch("lstm16_pack");
 }
 
-extern "C" int32_t stmgcn_lstm16_step_fwd(int32_t t, int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in,
-                                          int64_t b_inner, int32_t planes, const float* xo, const float* s_gate,
-                                          const void* const* wimg, const float* const* bias, const float* wih_t,
-                                          const void* h0p, const float* c0, void* hp, float* cs, float* h_top,
-                                          float* h_n, void* stream) {
-    STMGCN_REQUIRE(xo && s_gate && wimg && bias && wih_t && hp && cs, STMGCN_ERR_ARG, "lstm16_step_fwd: null pointer");
-    STMGCN_REQUIRE(planes == 1 || planes == 2, STMGCN_ERR_ARG, "lstm16_step_fwd: planes=%d", planes);
-    STMGCN_REQUIRE(t >= 0 && t < t_len && n_layers >= 1 && n_layers <= 8 && rows > 0 && c_in >= 1 && c_in <= kMaxC && b_inner > 0,
-                   STMGCN_ERR_SHAPE, "lstm16_step_fwd: t=%d T=%d L=%d rows=%lld C=%d", t, t_len, n_layers, (long long)rows, c_in);
-    STMGCN_REQUIRE(rows <= (1LL << 25), STMGCN_ERR_SHAPE, "lstm16_step_fwd: rows=%lld too large (32-bit element offsets)", (long long)rows);
-    STMGCN_REQUIRE((h0p == nullptr) == (c0 == nullptr), STMGCN_ERR_ARG, "lstm16_step_fwd: h0p and c0 go together");
+extern "C" int32_t stmgcn_lstm16_fwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in, int64_t b_inner,
+                                     int32_t planes, const float* xo, const float* s_gate, const void* const* wimg,
+                                     const float* const* bias, const float* wih_t, const void* h0p, const float* c0,
+                                     void* hp, float* cs, float* h_top, float* h_n, void* stream) {
+    STMGCN_REQUIRE(xo && s_gate && wimg && bias && wih_t && hp && cs, STMGCN_ERR_ARG, "lstm16_fwd: null pointer");
+    if (int32_t rc = check_args("lstm16_fwd", t_len, n_layers, rows, c_in, b_inner, planes, wimg, bias, h0p, c0)) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const int n_tiles = (int)ceil_div(rows, kTileM);
-    const int64_t rows_pad = (int64_t)n_tiles * kTileM;
     const int64_t plane_elems = rows * kHid;                       // bf16 elements per plane
-    const int64_t cslice = rows_pad * kHid;
+    const int64_t cslice = (int64_t)n_tiles * kTileM * kHid;
     const FwdFn fn0 = fwd_kernel_for(planes, c_in == 1 ? 1 : kMaxC), fn1 = fwd_kernel_for(planes, 0);
-    if (int32_t rc = set_smem_attr((const void*)fn0, kFSmem)) return rc;
-    if (int32_t rc = set_smem_attr((const void*)fn1, kFSmem)) return rc;
-    CUtensorMap hp_map, h0_map;
-    STMGCN_REQUIRE(make_plane_map(&hp_map, hp, rows, (int64_t)n_layers * t_len * planes), STMGCN_ERR_STATE,
-                   "lstm16_step_fwd: cuTensorMapEncodeTiled failed (hp)");
-    if (h0p != nullptr)
-        STMGCN_REQUIRE(make_plane_map(&h0_map, h0p, rows, (int64_t)n_layers * planes), STMGCN_ERR_STATE,
-                       "lstm16_step_fwd: cuTensorMapEncodeTiled failed (h0p)");
-    const int grid = n_tiles < sm_count() ? n_tiles : sm_count();
-    for (int l = 0; l < n_layers; ++l) {
-        STMGCN_REQUIRE(wimg[l] && bias[l], STMGCN_ERR_ARG, "lstm16_step_fwd: wimg/bias[%d] null", l);
-        Fwd16Params p;
-        memset(&p, 0, sizeof(p));
-        int ns = 0;
-        if (l > 0) {                                               // segment: h of the layer below at this step
-            p.amap[ns] = hp_map;
-            p.aslice[ns] = ((l - 1) * t_len + t) * planes;
-            ++ns;
+    if (int32_t rc = ensure_dyn_smem((const void*)fn0, kFSmem)) return rc;
+    if (int32_t rc = ensure_dyn_smem((const void*)fn1, kFSmem)) return rc;
+    CUtensorMap maps[2] = {};                                      // indexed by StepPlan::src: hp, h0p
+    if (int32_t rc = make_state_maps("lstm16_fwd", &maps[kSegHp], &maps[kSegH0], hp, h0p, rows, t_len, n_layers, planes))
+        return rc;
+    const int grid = grid_for(rows);
+    for (int t = 0; t < t_len; ++t)
+        for (int l = 0; l < n_layers; ++l) {
+            const StepPlan sp = plan_step(l, t, t_len, planes, c0, cs, cslice);
+            Fwd16Params p;
+            memset(&p, 0, sizeof(p));
+            for (int s = 0; s < sp.nseg; ++s)
+                if (sp.src[s] != kSegZero) {
+                    p.amap[p.nseg] = maps[sp.src[s]];
+                    p.aslice[p.nseg] = sp.slice[s];
+                    ++p.nseg;
+                }
+            p.wimg = (const uint8_t*)wimg[l];
+            p.bias = bias[l];
+            p.wih = (l == 0) ? wih_t : nullptr;
+            p.xo = xo;
+            p.sg = s_gate;
+            p.c_in = c_in;
+            p.t = t;
+            p.t_len = t_len;
+            p.b_inner = b_inner;
+            p.c_prev = sp.c_prev;
+            p.c_out = cs + (int64_t)(l * t_len + t) * cslice;
+            uint16_t* hbase = (uint16_t*)hp + (int64_t)(l * t_len + t) * planes * plane_elems;
+            p.h_hi = hbase;
+            p.h_lo = planes == 2 ? hbase + plane_elems : nullptr;
+            p.h_f32 = nullptr;
+            if (t == t_len - 1) {
+                if (h_n != nullptr) p.h_f32 = h_n + (int64_t)l * rows * kHid;
+                else if (l == n_layers - 1) p.h_f32 = h_top;
+            }
+            p.rows = rows;
+            p.n_tiles = n_tiles;
+            (l == 0 ? fn0 : fn1)<<<grid, kFThreads, kFSmem, st>>>(p);
+            count_launch();
+            if (int32_t rc = check_launch("lstm16_fwd")) return rc;
         }
-        if (t > 0) {                                               // segment: this layer's h of the previous step
-            p.amap[ns] = hp_map;
-            p.aslice[ns] = (l * t_len + t - 1) * planes;
-            ++ns;
-        } else if (h0p != nullptr) {
-            p.amap[ns] = h0_map;
-            p.aslice[ns] = l * planes;
-            ++ns;
-        }
-        p.nseg = ns;
-        // the weight image holds [seg0 hi | seg0 lo | seg1 hi | seg1 lo]; at t = 0 without h0 the h_prev segment is absent:
-        // layers > 0 then use only seg 0 (W_ih), layer 0 has no MMA at all
-        p.wimg = (const uint8_t*)wimg[l];
-        p.bias = bias[l];
-        p.wih = (l == 0) ? wih_t : nullptr;
-        p.xo = xo;
-        p.sg = s_gate;
-        p.c_in = c_in;
-        p.t = t;
-        p.t_len = t_len;
-        p.b_inner = b_inner;
-        p.c_prev = t > 0 ? cs + (int64_t)(l * t_len + t - 1) * cslice : (c0 ? c0 + (int64_t)l * cslice : nullptr);
-        p.c_out = cs + (int64_t)(l * t_len + t) * cslice;
-        uint16_t* hbase = (uint16_t*)hp + (int64_t)(l * t_len + t) * planes * plane_elems;
-        p.h_hi = hbase;
-        p.h_lo = planes == 2 ? hbase + plane_elems : nullptr;
-        p.h_f32 = nullptr;
-        if (t == t_len - 1) {
-            if (h_n != nullptr) p.h_f32 = h_n + (int64_t)l * rows * kHid;
-            else if (l == n_layers - 1) p.h_f32 = h_top;
-        }
-        p.rows = rows;
-        p.n_tiles = n_tiles;
-        (l == 0 ? fn0 : fn1)<<<grid, kFThreads, kFSmem, st>>>(p);
-        count_launch();
-        if (int32_t rc = check_launch("lstm16_fwd")) return rc;
-    }
     return 0;
 }
 
-extern "C" int32_t stmgcn_lstm16_grid(int64_t rows) {
-    const int64_t n_tiles = ceil_div(rows, kTileM);
-    return (int32_t)(n_tiles < sm_count() ? n_tiles : sm_count());
-}
+extern "C" int32_t stmgcn_lstm16_grid(int64_t rows) { return grid_for(rows); }
 
-extern "C" int32_t stmgcn_lstm16_layer_bwd(int32_t layer, int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in,
-                                           int64_t b_inner, int32_t planes, const float* xo, const float* s_gate,
-                                           const void* wimg, const float* bias, const float* wih_t, const void* h0p,
-                                           const float* c0, const void* hp, const float* cs, const float* dh_in,
-                                           float* dx_out, float* dh_rec, float* dc, float* d_s, float* dbp,
-                                           float* dw_scratch, const void* zero_tile, void* stream) {
-    STMGCN_REQUIRE(xo && s_gate && wimg && bias && hp && cs && dh_in && dh_rec && dc && d_s && dbp && dw_scratch && zero_tile,
-                   STMGCN_ERR_ARG, "lstm16_layer_bwd: null pointer");
-    STMGCN_REQUIRE(planes == 1 || planes == 2, STMGCN_ERR_ARG, "lstm16_layer_bwd: planes=%d", planes);
-    STMGCN_REQUIRE(layer >= 0 && layer < n_layers && n_layers <= 8 && t_len >= 1 && t_len <= kBMaxSteps && rows > 0 && c_in >= 1 &&
-                       c_in <= kMaxC && b_inner > 0,
-                   STMGCN_ERR_SHAPE, "lstm16_layer_bwd: layer=%d L=%d T=%d (max %d) rows=%lld C=%d", layer, n_layers, t_len,
-                   kBMaxSteps, (long long)rows, c_in);
-    STMGCN_REQUIRE(rows <= (1LL << 25), STMGCN_ERR_SHAPE, "lstm16_layer_bwd: rows=%lld too large (32-bit element offsets)", (long long)rows);
-    STMGCN_REQUIRE((h0p == nullptr) == (c0 == nullptr), STMGCN_ERR_ARG, "lstm16_layer_bwd: h0p and c0 go together");
-    STMGCN_REQUIRE((layer == 0) == (dx_out == nullptr), STMGCN_ERR_ARG, "lstm16_layer_bwd: dx_out is for layers > 0 only");
-    STMGCN_REQUIRE(layer > 0 || wih_t != nullptr, STMGCN_ERR_ARG, "lstm16_layer_bwd: wih_t null");
+extern "C" int32_t stmgcn_lstm16_bwd(int32_t t_len, int32_t n_layers, int64_t rows, int32_t c_in, int64_t b_inner,
+                                     int32_t planes, const float* xo, const float* s_gate, const void* const* wimg,
+                                     const float* const* bias, const float* wih_t, const void* h0p, const float* c0,
+                                     const void* hp, const float* cs, const float* d_top, float* dh_rec, float* dc,
+                                     float* dx_work, float* d_s, float* dbp, float* dw_scratch, const void* zero_tile,
+                                     float* const* grads, void* stream) {
+    STMGCN_REQUIRE(xo && s_gate && wimg && bias && wih_t && hp && cs && d_top && dh_rec && dc && d_s && dbp && dw_scratch &&
+                       zero_tile && grads,
+                   STMGCN_ERR_ARG, "lstm16_bwd: null pointer");
+    if (int32_t rc = check_args("lstm16_bwd", t_len, n_layers, rows, c_in, b_inner, planes, wimg, bias, h0p, c0)) return rc;
+    STMGCN_REQUIRE(t_len <= kBMaxSteps, STMGCN_ERR_SHAPE, "lstm16_bwd: T=%d (max %d)", t_len, kBMaxSteps);
+    STMGCN_REQUIRE((n_layers > 1) == (dx_work != nullptr), STMGCN_ERR_ARG, "lstm16_bwd: dx_work is needed exactly when L > 1 (L=%d)",
+                   n_layers);
+    for (int i = 0; i < 4 * n_layers; ++i) STMGCN_REQUIRE(grads[i], STMGCN_ERR_ARG, "lstm16_bwd: grads[%d] null", i);
     cudaStream_t st = (cudaStream_t)stream;
     const int n_tiles = (int)ceil_div(rows, kTileM);
     const int64_t cslice = (int64_t)n_tiles * kTileM * kHid;
-    const int l = layer;
-    const BwdFn fn = bwd_kernel_for(planes, l == 0 ? (c_in == 1 ? 1 : kMaxC) : 0);
-    if (int32_t rc = set_smem_attr((const void*)fn, kBSmem)) return rc;
-    Bwd16Params p;
-    memset(&p, 0, sizeof(p));
-    STMGCN_REQUIRE(make_plane_map(&p.maps[0], hp, rows, (int64_t)n_layers * t_len * planes), STMGCN_ERR_STATE,
-                   "lstm16_layer_bwd: cuTensorMapEncodeTiled failed (hp)");
-    if (h0p != nullptr)
-        STMGCN_REQUIRE(make_plane_map(&p.maps[1], h0p, rows, (int64_t)n_layers * planes), STMGCN_ERR_STATE,
-                       "lstm16_layer_bwd: cuTensorMapEncodeTiled failed (h0p)");
-    const int grid = n_tiles < sm_count() ? n_tiles : sm_count();
-    const bool top = (l == n_layers - 1);
-    p.zero_tile = (const uint8_t*)zero_tile;
-    p.wimg = (const uint8_t*)wimg;
-    p.bias = bias;
-    p.wih = (l == 0) ? wih_t : nullptr;
-    p.xo = xo;
-    p.sg = s_gate;
-    p.d_s = d_s;
-    p.c_in = c_in;
-    p.t_len = t_len;
-    p.b_inner = b_inner;
-    p.dh_rec = dh_rec;
-    p.dc = dc;
-    p.dbp = dbp;
-    p.dw_slice = dw_scratch;
-    p.rows = rows;
-    p.n_tiles = n_tiles;
+    CUtensorMap maps[2] = {};                                      // Bwd16Params::maps: hp, h0p
+    if (int32_t rc = make_state_maps("lstm16_bwd", &maps[kSegHp], &maps[kSegH0], hp, h0p, rows, t_len, n_layers, planes))
+        return rc;
+    const int grid = grid_for(rows);
+    const int64_t wg_slices = (int64_t)grid * (kTileM * kGateCols);  // one layer's dw_scratch
     // Steps per launch: the weight-gradient accumulator of a CTA lives in TMEM for the whole launch, and the tensor core's fp32
     // accumulation loses precision with the length of the chain (all T steps of cfg5's 7 tiles per CTA = 21.5 k rows in one
     // chain put 1.3e-4 into the LSTM weight gradients, measured; per-step launches, 1.8 k rows: 1.4e-5).  A launch therefore
@@ -1325,53 +1328,68 @@ extern "C" int32_t stmgcn_lstm16_layer_bwd(int32_t layer, int32_t t_len, int32_t
     const int tiles_per_cta = (int)ceil_div(n_tiles, grid);
     int steps_per_launch = kMaxChainItems / tiles_per_cta;
     if (steps_per_launch < 1) steps_per_launch = 1;
-    for (int s0 = 0; s0 < t_len; s0 += steps_per_launch) {
-        const int ns_launch = (t_len - s0 < steps_per_launch) ? (t_len - s0) : steps_per_launch;
-        p.n_steps = ns_launch;
-        p.dw_first = (s0 == 0) ? 1 : 0;
-        for (int sj = 0; sj < ns_launch; ++sj) {
-            const int si = s0 + sj;
-            const int t = t_len - 1 - si;
-            Bwd16Step& sp = p.steps[sj];
-            int ns = 0;
-            if (l > 0) {                                               // K segment: h of the layer below at this step
-                sp.src[ns] = 0;
-                sp.slice[ns] = ((l - 1) * t_len + t) * planes;
-                ++ns;
+    // Layers top-down.  A layer reads the gradient of its output from the layer above -- the top layer d_top at T-1 only --
+    // and writes the gradient of its input (dx, every step) for the layer below: two slices of dx_work alternate.
+    const float* dh_in = d_top;
+    for (int l = n_layers - 1; l >= 0; --l) {
+        const bool top = (l == n_layers - 1);
+        float* dx_out = l > 0 ? dx_work + (int64_t)((n_layers - 1 - l) % 2) * t_len * cslice : nullptr;
+        const BwdFn fn = bwd_kernel_for(planes, l == 0 ? (c_in == 1 ? 1 : kMaxC) : 0);
+        if (int32_t rc = ensure_dyn_smem((const void*)fn, kBSmem)) return rc;
+        Bwd16Params p;
+        memset(&p, 0, sizeof(p));
+        p.maps[0] = maps[0];
+        p.maps[1] = maps[1];
+        p.zero_tile = (const uint8_t*)zero_tile;
+        p.wimg = (const uint8_t*)wimg[l];
+        p.bias = bias[l];
+        p.wih = (l == 0) ? wih_t : nullptr;
+        p.xo = xo;
+        p.sg = s_gate;
+        p.d_s = d_s;
+        p.c_in = c_in;
+        p.t_len = t_len;
+        p.b_inner = b_inner;
+        p.dh_rec = dh_rec;
+        p.dc = dc;
+        p.dbp = dbp + (int64_t)l * kGateCols;
+        p.dw_slice = dw_scratch + l * wg_slices;
+        p.rows = rows;
+        p.n_tiles = n_tiles;
+        for (int s0 = 0; s0 < t_len; s0 += steps_per_launch) {
+            const int ns_launch = (t_len - s0 < steps_per_launch) ? (t_len - s0) : steps_per_launch;
+            p.n_steps = ns_launch;
+            p.dw_first = (s0 == 0) ? 1 : 0;
+            for (int sj = 0; sj < ns_launch; ++sj) {
+                const int t = t_len - 1 - (s0 + sj);
+                const StepPlan plan = plan_step(l, t, t_len, planes, c0, cs, cslice);
+                Bwd16Step& sp = p.steps[sj];
+                for (int s = 0; s < 2; ++s) {
+                    sp.src[s] = plan.src[s];
+                    sp.slice[s] = plan.slice[s];
+                }
+                sp.t = t;
+                sp.first = (t == t_len - 1) ? 1 : 0;
+                sp.store_dh = (t > 0 || h0p != nullptr) ? 1 : 0;
+                sp.c_prev = plan.c_prev;
+                sp.dh_in = top ? (t == t_len - 1 ? dh_in : nullptr) : dh_in + (int64_t)t * cslice;
+                sp.dx_out = l > 0 ? dx_out + (int64_t)t * cslice : nullptr;
             }
-            if (t > 0) {                                               // K segment: this layer's h of the previous step
-                sp.src[ns] = 0;
-                sp.slice[ns] = (l * t_len + t - 1) * planes;
-            } else if (h0p != nullptr) {
-                sp.src[ns] = 1;
-                sp.slice[ns] = l * planes;
-            } else {
-                sp.src[ns] = 2;                                        // zeros (STMGCN.py:53-57)
-                sp.slice[ns] = 0;
-            }
-            sp.t = t;
-            sp.first = (t == t_len - 1) ? 1 : 0;
-            sp.store_dh = (t > 0 || h0p != nullptr) ? 1 : 0;
-            sp.c_prev = t > 0 ? cs + (int64_t)(l * t_len + t - 1) * cslice : (c0 ? c0 + (int64_t)l * cslice : nullptr);
-            sp.dh_in = top ? (t == t_len - 1 ? dh_in : nullptr) : dh_in + (int64_t)t * cslice;
-            sp.dx_out = l > 0 ? dx_out + (int64_t)t * cslice : nullptr;
+            fn<<<grid, kBThreads, kBSmem, st>>>(p);
+            count_launch();
+            if (int32_t rc = check_launch("lstm16_bwd")) return rc;
         }
-        fn<<<grid, kBThreads, kBSmem, st>>>(p);
+        dh_in = dx_out;
+    }
+    // per layer: sum the CTAs' scratch slices into the nn.LSTM-native gradients w_ih, w_hh, b_ih, b_hh
+    for (int l = 0; l < n_layers; ++l) {
+        float* const* g = grads + 4 * l;
+        lstm16_wgrad_reduce_kernel<<<(kTileM * kGateCols) / 256, 256, 0, st>>>(dw_scratch + l * wg_slices, grid, l, c_in,
+                                                                             dbp + (int64_t)l * kGateCols, g[0], g[1], g[2], g[3]);
         count_launch();
-        if (int32_t rc = check_launch("lstm16_layer_bwd")) return rc;
+        if (int32_t rc = check_launch("lstm16_bwd (weight-gradient reduction)")) return rc;
     }
     return 0;
-}
-
-extern "C" int32_t stmgcn_lstm16_wgrad_reduce(int32_t layer, int32_t c_in, int32_t n_slices, const float* slices,
-                                              const float* dbp, float* d_w_ih, float* d_w_hh, float* d_b_ih,
-                                              float* d_b_hh, void* stream) {
-    STMGCN_REQUIRE(slices && dbp && d_w_ih && d_w_hh && d_b_ih && d_b_hh, STMGCN_ERR_ARG, "lstm16_wgrad_reduce: null pointer");
-    STMGCN_REQUIRE(layer >= 0 && n_slices >= 1 && c_in >= 1 && c_in <= kMaxC, STMGCN_ERR_SHAPE, "lstm16_wgrad_reduce: bad sizes");
-    lstm16_wgrad_reduce_kernel<<<(kTileM * kGateCols) / 256, 256, 0, (cudaStream_t)stream>>>(slices, n_slices, layer, c_in, dbp,
-                                                                                        d_w_ih, d_w_hh, d_b_ih, d_b_hh);
-    count_launch();
-    return check_launch("lstm16_wgrad_reduce");
 }
 
 #ifdef STMGCN_TC_PROFILE

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("STMGCN_LIB_PATH") or os.path.join(os.path.dirname(_HERE), "lib", "libstmgcn_b200.so")
 
 ACT_NONE, ACT_RELU = 0, 1
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 # (name, restype, argtypes) -- one row per symbol in include/stmgcn_b200.h
 _P = c_void_p
@@ -42,19 +42,18 @@ SIGNATURES = [
                                      _P]),
     ("stmgcn_gate_fwd", c_int32, [_P, c_int64, c_int32, c_int64, _P, _P, _P, _P, _P, _P]),
     ("stmgcn_gate_bwd", c_int32, [_P, _P, _P, _P, c_int64, c_int32, _P, _P, _P, _P, _P]),
-    ("stmgcn_lstm_step_fwd", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, c_int32, c_int64, _P, _P,
-                                       _P, POINTER(c_void_p), POINTER(c_void_p), _P, _P, _P, _P, _P, _P]),
-    ("stmgcn_lstm_step_bwd", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, c_int32, c_int64, _P, _P,
-                                       _P, POINTER(c_void_p), _P, _P, _P, _P, _P, _P, _P, _P, _P,
-                                       POINTER(c_void_p), _P]),
-    ("stmgcn_lstm_wgrad", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, _P, _P, _P, _P, _P]),
+    ("stmgcn_lstm_fwd", c_int32, [c_int32, c_int32, c_int64, c_int32, c_int32, c_int64, _P, _P, _P,
+                                  POINTER(c_void_p), POINTER(c_void_p), _P, _P, _P, _P, _P, _P]),
+    ("stmgcn_lstm_bwd", c_int32, [c_int32, c_int32, c_int64, c_int32, c_int32, c_int64, _P, _P, _P,
+                                  POINTER(c_void_p), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                  POINTER(c_void_p), POINTER(c_void_p), _P]),
     ("stmgcn_lstm16_pack", c_int32, [_P, _P, _P, _P, c_int32, c_int32, _P, _P, _P, _P]),
-    ("stmgcn_lstm16_step_fwd", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, c_int64, c_int32, _P, _P,
-                                         POINTER(c_void_p), POINTER(c_void_p), _P, _P, _P, _P, _P, _P, _P, _P]),
+    ("stmgcn_lstm16_fwd", c_int32, [c_int32, c_int32, c_int64, c_int32, c_int64, c_int32, _P, _P,
+                                    POINTER(c_void_p), POINTER(c_void_p), _P, _P, _P, _P, _P, _P, _P, _P]),
     ("stmgcn_lstm16_grid", c_int32, [c_int64]),
-    ("stmgcn_lstm16_layer_bwd", c_int32, [c_int32, c_int32, c_int32, c_int64, c_int32, c_int64, c_int32, _P, _P,
-                                          _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
-    ("stmgcn_lstm16_wgrad_reduce", c_int32, [c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, _P, _P]),
+    ("stmgcn_lstm16_bwd", c_int32, [c_int32, c_int32, c_int64, c_int32, c_int64, c_int32, _P, _P,
+                                    POINTER(c_void_p), POINTER(c_void_p), _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                    _P, _P, _P, POINTER(c_void_p), _P]),
     ("stmgcn_fuse_out_fwd", c_int32, [POINTER(c_void_p), c_int32, c_int64, c_int64, c_int32, c_int32, _P, _P,
                                       _P, _P, _P]),
     ("stmgcn_fuse_out_bwd", c_int32, [_P, _P, c_int64, c_int64, c_int32, c_int32, _P, _P, _P, _P, _P]),

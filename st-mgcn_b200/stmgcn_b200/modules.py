@@ -89,7 +89,7 @@ class CG_LSTM(nn.Module):
                                         bias=gconv_use_bias, activation=gconv_activation)
         self.fc = nn.Linear(in_features=seq_len, out_features=seq_len, bias=True)
         # nn.LSTM is kept as the PARAMETER CONTAINER only (names weight_ih_l0 ... as in the reference);
-        # its forward is never called -- the recurrence runs in stmgcn_lstm_step_fwd/bwd.
+        # its forward is never called -- the recurrence runs in ops.SharedLSTM (stmgcn_lstm16_fwd/bwd, stmgcn_lstm_fwd/bwd).
         self.lstm = nn.LSTM(input_size=input_dim, hidden_size=lstm_hidden_dim,
                             num_layers=lstm_num_layers, batch_first=True)
 

@@ -495,10 +495,11 @@ def _lstm_inputs(xo, s_gate, h0, c0, weights):
 
 
 class SharedLSTM16(torch.autograd.Function):
-    """:class:`SharedLSTM` on the tcgen05 bf16-plane kernels of lstm16.cu (H = 64, C <= 4, T <= 64).  Tape: the hidden
-    states as bf16 planes plus the cell state, no gate tape.  The backward recomputes the gates: ONE fused launch per
-    layer over all timesteps (gate recompute + pointwise + data gradient + weight gradient, stmgcn_lstm16_layer_bwd),
-    layers top-down, then one reduction per layer."""
+    """:class:`SharedLSTM` on the tcgen05 bf16-plane kernels of lstm16.cu (H = 64, C <= 4, T <= 64), one library call
+    per direction (stmgcn_lstm16_fwd / _bwd run the whole recurrence).  Tape: the hidden states as bf16 planes plus the
+    cell state, no gate tape.  The backward recomputes the gates in fused launches (gate recompute + pointwise + data
+    gradient + weight gradient), each covering one layer and a run of timesteps -- up to ceil(T / steps per launch) per
+    layer, layers top-down -- then one reduction per layer."""
 
     @staticmethod
     def forward(ctx, xo, s_gate, h0, c0, n_layers: int, hid: int, want_state: bool, *weights):
@@ -519,12 +520,9 @@ class SharedLSTM16(torch.autograd.Function):
         else:
             h_n = None
             h_top = torch.empty((rows, 64), device=dev, dtype=torch.float32)
-        st = _stream()
-        for t in range(t_len):
-            _lib.check(L.stmgcn_lstm16_step_fwd(t, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
-                                                img["wimg_arr"], img["bias_arr"], img["wih_t"].data_ptr(), _p(h0p), _p(c0b),
-                                                hp.data_ptr(), cs.data_ptr(), h_top.data_ptr(), _p(h_n), st),
-                       "lstm16_step_fwd")
+        _lib.check(L.stmgcn_lstm16_fwd(t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
+                                       img["wimg_arr"], img["bias_arr"], img["wih_t"].data_ptr(), _p(h0p), _p(c0b),
+                                       hp.data_ptr(), cs.data_ptr(), h_top.data_ptr(), _p(h_n), _stream()), "lstm16_fwd")
         if want_state:
             c_n = from_blocked(cs[:, t_len - 1], rows)
         else:
@@ -550,40 +548,31 @@ class SharedLSTM16(torch.autograd.Function):
         d_top_b = to_blocked(_f32c(d_top).view(rows, 64))
         dh_rec = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
         dc = torch.empty((rows_pad, 64), device=dev, dtype=torch.float32)
-        # dx of a layer for every timestep: written by layer l, read by layer l - 1 (two buffers ping-pong down the stack)
-        dx_bufs = [torch.empty((t_len, rows_pad, 64), device=dev, dtype=torch.float32) for _ in range(min(2, n_layers - 1))]
+        # the gradient a layer passes to the layer below, every timestep (two slices alternate down the stack)
+        dx_work = (torch.empty((min(2, n_layers - 1), t_len, rows_pad, 64), device=dev, dtype=torch.float32)
+                   if n_layers > 1 else None)
         d_s = torch.zeros((b, t_len), device=dev, dtype=torch.float32)
         dbp = torch.zeros((n_layers, 256), device=dev, dtype=torch.float32)
-        grid = int(L.stmgcn_lstm16_grid(rows))
-        scratch = torch.empty((n_layers, grid, 128 * 256), device=dev, dtype=torch.float32)
-        zero = _zero_tile(dev)
-        st = _stream()
-        dh_in = d_top_b
-        for l in range(n_layers - 1, -1, -1):
-            dx_out = dx_bufs[(n_layers - 1 - l) % 2] if l > 0 else None
-            _lib.check(L.stmgcn_lstm16_layer_bwd(l, t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
-                                                 img["wimg"][l].data_ptr(), img["bias"][l].data_ptr(), img["wih_t"].data_ptr(),
-                                                 _p(tape["h0p"]), _p(tape["c0b"]), tape["hp"].data_ptr(), tape["cs"].data_ptr(),
-                                                 dh_in.data_ptr(), _p(dx_out), dh_rec.data_ptr(), dc.data_ptr(), d_s.data_ptr(),
-                                                 dbp[l].data_ptr(), scratch[l].data_ptr(), zero.data_ptr(), st), "lstm16_layer_bwd")
-            dh_in = dx_out
+        scratch = torch.empty((n_layers, int(L.stmgcn_lstm16_grid(rows)), 128 * 256), device=dev, dtype=torch.float32)
         w_grads = []
         for l in range(n_layers):
             in_l = c_in if l == 0 else 64
-            d_w_ih = torch.empty((256, in_l), device=dev, dtype=torch.float32)
-            d_w_hh = torch.empty((256, 64), device=dev, dtype=torch.float32)
-            d_b_ih = torch.empty(256, device=dev, dtype=torch.float32)
-            d_b_hh = torch.empty(256, device=dev, dtype=torch.float32)
-            _lib.check(L.stmgcn_lstm16_wgrad_reduce(l, c_in, grid, scratch[l].data_ptr(), dbp[l].data_ptr(), d_w_ih.data_ptr(),
-                                                    d_w_hh.data_ptr(), d_b_ih.data_ptr(), d_b_hh.data_ptr(), st),
-                       "lstm16_wgrad_reduce")
-            w_grads += [d_w_ih, d_w_hh, d_b_ih, d_b_hh]
+            w_grads += [torch.empty((256, in_l), device=dev, dtype=torch.float32),
+                        torch.empty((256, 64), device=dev, dtype=torch.float32),
+                        torch.empty(256, device=dev, dtype=torch.float32), torch.empty(256, device=dev, dtype=torch.float32)]
+        _lib.check(L.stmgcn_lstm16_bwd(t_len, n_layers, rows, c_in, b, planes, xo.data_ptr(), s_gate.data_ptr(),
+                                       img["wimg_arr"], img["bias_arr"], img["wih_t"].data_ptr(), _p(tape["h0p"]),
+                                       _p(tape["c0b"]), tape["hp"].data_ptr(), tape["cs"].data_ptr(), d_top_b.data_ptr(),
+                                       dh_rec.data_ptr(), dc.data_ptr(), _p(dx_work), d_s.data_ptr(), dbp.data_ptr(),
+                                       scratch.data_ptr(), _zero_tile(dev).data_ptr(),
+                                       _lib.ptr_array([g.data_ptr() for g in w_grads]), _stream()), "lstm16_bwd")
         return (None, d_s, None, None, None, None, None, *w_grads)
 
 
 class SharedLSTMExact(torch.autograd.Function):
-    """:class:`SharedLSTM` on the exact-fp32 CUDA-core kernels of lstm.cu (any H <= 128).  Tape: hs, cs and the
-    post-activation gates; the backward overwrites the gate tape in place, so it can run only once per forward."""
+    """:class:`SharedLSTM` on the exact-fp32 CUDA-core kernels of lstm.cu (any H <= 128), one library call per direction
+    (stmgcn_lstm_fwd / _bwd).  Tape: hs, cs and the post-activation gates; the backward overwrites the gate tape in
+    place, so it can run only once per forward."""
 
     @staticmethod
     def forward(ctx, xo, s_gate, h0, c0, n_layers: int, hid: int, want_state: bool, *weights):
@@ -597,11 +586,9 @@ class SharedLSTMExact(torch.autograd.Function):
         cs = torch.empty((n_layers, t_len, rows, hid), device=dev, dtype=torch.float32)
         gates = torch.empty((n_layers, t_len, rows, 4 * hid), device=dev, dtype=torch.float32) if need_grad else None
         wp_arr, bp_arr = _lib.ptr_array([w.data_ptr() for w in wp]), _lib.ptr_array([v.data_ptr() for v in bp])
-        st = _stream()
-        for t in range(t_len):
-            _lib.check(L.stmgcn_lstm_step_fwd(t, t_len, n_layers, rows, hid, c_in, b, xo.data_ptr(),
-                                              s_gate.data_ptr(), wx.data_ptr(), wp_arr, bp_arr, _p(h0), _p(c0),
-                                              hs.data_ptr(), cs.data_ptr(), _p(gates), st), "lstm_step_fwd")
+        _lib.check(L.stmgcn_lstm_fwd(t_len, n_layers, rows, hid, c_in, b, xo.data_ptr(), s_gate.data_ptr(), wx.data_ptr(),
+                                     wp_arr, bp_arr, _p(h0), _p(c0), hs.data_ptr(), cs.data_ptr(), _p(gates), _stream()),
+                   "lstm_fwd")
         if need_grad:
             ctx.dims = (n, b, t_len, c_in, n_layers, hid)
             ctx.save_for_backward(xo, s_gate, h0, c0, hs, cs, gates, wx, *wpt)
@@ -624,7 +611,7 @@ class SharedLSTMExact(torch.autograd.Function):
         rows = n * b
         dev = xo.device
         d_top = _f32c(d_top).view(rows, hid)
-        # dh_rec / dc need no initialisation: the step at t = T-1 treats them as zero (stmgcn_lstm_step_bwd)
+        # dh_rec / dc need no initialisation: the step at t = T-1 treats them as zero (stmgcn_lstm_bwd)
         dh_rec = torch.empty((n_layers, rows, hid), device=dev, dtype=torch.float32)
         dc = torch.empty((n_layers, rows, hid), device=dev, dtype=torch.float32)
         dx_work = torch.empty((rows, hid), device=dev, dtype=torch.float32)
@@ -632,19 +619,12 @@ class SharedLSTMExact(torch.autograd.Function):
         dwx = torch.zeros_like(wx)
         dbp = [torch.zeros(4 * hid, device=dev, dtype=torch.float32) for _ in range(n_layers)]
         dwp = [torch.zeros((w.shape[1], 4 * hid), device=dev, dtype=torch.float32) for w in wpt]
-        wpt_arr = _lib.ptr_array([w.data_ptr() for w in wpt])
-        dbp_arr = _lib.ptr_array([v.data_ptr() for v in dbp])
-        st = _stream()
+        wpt_arr, dbp_arr, dwp_arr = (_lib.ptr_array([v.data_ptr() for v in ts]) for ts in (wpt, dbp, dwp))
         # NOTE: gates is overwritten in place with dA (the tape is consumed; see the guard above)
-        for t in range(t_len - 1, -1, -1):
-            _lib.check(L.stmgcn_lstm_step_bwd(t, t_len, n_layers, rows, hid, c_in, b, xo.data_ptr(),
-                                              s_gate.data_ptr(), wx.data_ptr(), wpt_arr, _p(c0), cs.data_ptr(),
-                                              gates.data_ptr(), d_top.data_ptr(), dh_rec.data_ptr(),
-                                              dc.data_ptr(), dx_work.data_ptr(), d_s.data_ptr(), dwx.data_ptr(),
-                                              dbp_arr, st), "lstm_step_bwd")
-        for l in range(n_layers):
-            _lib.check(L.stmgcn_lstm_wgrad(l, t_len, n_layers, rows, hid, _p(h0), hs.data_ptr(), gates.data_ptr(),
-                                           dwp[l].data_ptr(), st), "lstm_wgrad")
+        _lib.check(L.stmgcn_lstm_bwd(t_len, n_layers, rows, hid, c_in, b, xo.data_ptr(), s_gate.data_ptr(), wx.data_ptr(),
+                                     wpt_arr, _p(h0), _p(c0), hs.data_ptr(), cs.data_ptr(), gates.data_ptr(),
+                                     d_top.data_ptr(), dh_rec.data_ptr(), dc.data_ptr(), dx_work.data_ptr(), d_s.data_ptr(),
+                                     dwx.data_ptr(), dbp_arr, dwp_arr, _stream()), "lstm_bwd")
         w_grads = _unpack_lstm_grads(dwx, dwp, dbp, n_layers, hid, c_in)
         return (None, d_s, None, None, None, None, None, *w_grads)
 

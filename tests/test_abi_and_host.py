@@ -39,7 +39,8 @@ def test_library_exports_every_declared_symbol():
 
 def test_c_abi_argument_errors_come_back_as_codes_with_a_message():
     """The C entry points validate their arguments before touching CUDA: a bad call returns a negative code and
-    stmgcn_last_error() explains it (no GPU needed).  Covers the entries added in ABI 3 and 4."""
+    stmgcn_last_error() explains it (no GPU needed).  Covers the entries added in ABI 3 and 4 (the LSTM's: see
+    test_lstm_entries_reject_bad_arguments_before_any_cuda_call)."""
     import ctypes
     from stmgcn_b200 import _lib
     lib = _lib.lib
@@ -58,15 +59,51 @@ def test_c_abi_argument_errors_come_back_as_codes_with_a_message():
     for name, call, null_arg in (("proj_fwd_tc", fwd_tc, "out"), ("proj_bwd_tc", bwd_tc, "u")):
         for kwargs, code in (({"ks": 9}, err_shape), ({null_arg: null}, err_arg), ({"s": odd}, err_align)):
             assert call(**kwargs) == code and name.encode() in lib.stmgcn_last_error(), (name, kwargs)
-    # time-fused LSTM backward: null workspaces
-    rc = lib.stmgcn_lstm16_layer_bwd(0, 12, 3, 128, 1, 8, 2, *([null] * 18))
-    assert rc < 0 and b"lstm16_layer_bwd" in lib.stmgcn_last_error()
     # bf16 gather step: null graph; conversion: count not a multiple of 8
     rc = lib.stmgcn_cheb_spmm_step16(null, 0, 1.0, null, 0.0, null, 0.0, null, null, null, 64, null)
     assert rc < 0 and b"cheb_spmm_step16" in lib.stmgcn_last_error()
     buf = (ctypes.c_float * 16)()
     rc = lib.stmgcn_to_bf16(ctypes.addressof(buf), ctypes.addressof(buf), 12, null)
     assert rc < 0 and b"multiple of 8" in lib.stmgcn_last_error()
+
+
+def test_lstm_entries_reject_bad_arguments_before_any_cuda_call():
+    """One LSTM entry per kernel family and direction runs the whole recurrence (ABI 5).  Each rejects a null required
+    pointer (ERR_ARG), a shape out of range (ERR_SHAPE) and, in the backward, a missing dx workspace with L > 1 (ERR_ARG),
+    with a message naming the entry -- before any CUDA call (no GPU needed; the fake device pointers are never read)."""
+    import ctypes
+    from stmgcn_b200 import _lib
+    lib = _lib.lib
+    null, ok = ctypes.c_void_p(0), ctypes.c_void_p(256)
+    err_arg, err_shape = -1, -2
+    n_layers, t_len, rows, c_in, b_inner, hid = 3, 12, 128, 1, 8, 64
+
+    def arr(n):
+        return _lib.ptr_array([256] * n)
+
+    def lstm16_fwd(c=c_in, xo=ok):
+        return lib.stmgcn_lstm16_fwd(t_len, n_layers, rows, c, b_inner, 2, xo, ok, arr(n_layers), arr(n_layers), ok, null,
+                                     null, ok, ok, ok, null, null)
+
+    def lstm16_bwd(t=t_len, cs=ok, dx_work=ok):
+        return lib.stmgcn_lstm16_bwd(t, n_layers, rows, c_in, b_inner, 2, ok, ok, arr(n_layers), arr(n_layers), ok, null,
+                                     null, ok, cs, ok, ok, ok, dx_work, ok, ok, ok, ok, arr(4 * n_layers), null)
+
+    def lstm_fwd(h=hid, hs=ok):
+        return lib.stmgcn_lstm_fwd(t_len, n_layers, rows, h, c_in, b_inner, ok, ok, ok, arr(n_layers), arr(n_layers), null,
+                                   null, hs, ok, null, null)
+
+    def lstm_bwd(h=hid, gates=ok, dx_work=ok):
+        return lib.stmgcn_lstm_bwd(t_len, n_layers, rows, h, c_in, b_inner, ok, ok, ok, arr(n_layers), null, null, ok, ok,
+                                   gates, ok, ok, ok, dx_work, ok, ok, arr(n_layers), arr(n_layers), null)
+
+    for name, call, cases in (
+            ("lstm16_fwd", lstm16_fwd, (({"xo": null}, err_arg), ({"c": 5}, err_shape))),
+            ("lstm16_bwd", lstm16_bwd, (({"cs": null}, err_arg), ({"t": 65}, err_shape), ({"dx_work": null}, err_arg))),
+            ("lstm_fwd", lstm_fwd, (({"hs": null}, err_arg), ({"h": 130}, err_shape))),
+            ("lstm_bwd", lstm_bwd, (({"gates": null}, err_arg), ({"h": 130}, err_shape), ({"dx_work": null}, err_arg)))):
+        for kwargs, code in cases:
+            assert call(**kwargs) == code and name.encode() + b":" in lib.stmgcn_last_error(), (name, kwargs)
 
 
 def test_no_cpu_fallback_is_loud():
@@ -175,7 +212,7 @@ def test_lstm_weight_packing_roundtrip():
 @pytest.mark.parametrize("rows", [128, 300, 1])
 def test_tile_blocked_layout_roundtrip_and_formula(rows):
     """to_blocked / from_blocked are inverse, pad to whole 128-row tiles, and place element (r, u) where the kernels'
-    ws_off() expects it: (((r/128)*16 + u/4)*128 + r%128)*4 + u%4  (include/stmgcn_b200.h, stmgcn_lstm16_step_fwd)."""
+    ws_off() expects it: (((r/128)*16 + u/4)*128 + r%128)*4 + u%4  (include/stmgcn_b200.h, stmgcn_lstm16_fwd)."""
     from stmgcn_b200 import ops
     gen = torch.Generator().manual_seed(rows)
     x = torch.randn(2, rows, 64, generator=gen)
